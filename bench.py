@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the loss-head hot path (BASELINE.json metric: DPO pair-tokens/s fwd+bwd; NT-Xent pairs/s as extras).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload at every N (weak scaling, one process per GPU): BASELINE config 2 — Stage-2 DPO head, GPT-2 Medium LM head
 (d=1024, V=50257), 16 preference pairs per GPU, seq 128, beta=0.1, random-init weights, synthetic hidden states.
@@ -14,6 +14,8 @@ A pair-token is one scored position of one (chosen, rejected) pair: B*(T-1) = 20
 `roofline` the dominant kernel of the step against the measured bf16 tensor-core peak (MEASURED_PEAKS.json).
 `cpu_baseline` the reference's CPU path (oracle/torch_port.py) timed on this box's host cores, bounded sample.
 `--impl reference` times that CPU path alone, on all host threads, in the same JSON shape.
+`--dump-outputs DIR` writes what the last timed resident step returned (rank 0) to DIR/<name>.npy, float32; the inputs
+          are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -239,6 +241,25 @@ def run_reference(args, rank):
 
 
 # ----------------------------------------------------------------------------------------------- our arm
+DUMP_DW_ROW_STRIDE = 8  # dW is V x d fp32 (206 MB): every 8th vocabulary row keeps the dump within 64 MB
+
+
+def dump_outputs(path, outputs):
+    """What one resident step hands back, as float32 .npy files under `path`: the sequence log-probs of both forwards,
+    the DPO loss and metrics, dH in full and dW sampled every DUMP_DW_ROW_STRIDE-th row (rows 0, 8, 16, ...)."""
+    import numpy as np
+    seq_p, seq_r, loss, metrics, dh, dw = outputs
+    arrays = {"policy_seq_logprobs": seq_p, "reference_seq_logprobs": seq_r, "loss": loss, "metrics": metrics,
+              "dhidden": dh, f"dweight_rows_stride{DUMP_DW_ROW_STRIDE}": dw[::DUMP_DW_ROW_STRIDE]}
+    arrays = {name: t.detach().float().cpu().numpy() for name, t in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"output dump of {total} bytes exceeds 64 MB"
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    log(f"dumped {len(arrays)} outputs of the last timed step ({total / 2 ** 20:.1f} MB) to {path}")
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -306,7 +327,7 @@ def run_ours(args, rank, world, local_rank):
             mark(5)
             torch.cuda.current_stream().wait_event(done)  # dW (and the scalars) summed over the ranks
             mark(6)
-            return packed[0], dh, dw
+            return seq_p, seq_r, packed[0], packed[1:], dh, dw
         if fused:
             dh, dw = F.lmhead_logprob_bwd(H, W, rl, rw, lse_p, gseq, False)
             mark(4)
@@ -321,7 +342,8 @@ def run_ours(args, rank, world, local_rank):
             packed = torch.cat([loss.reshape(1), metrics])
             dist.all_reduce(packed)
             mark(6)
-        return loss, dh, dw
+            loss, metrics = packed[0], packed[1:]
+        return seq_p, seq_r, loss, metrics, dh, dw
 
     for _ in range(max(args.warmup, 3)):
         resident_step()
@@ -333,13 +355,17 @@ def run_ours(args, rank, world, local_rank):
     t_begin, t_end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     t_begin.record()
-    for k in range(args.steps):
+    for k in range(args.steps - 1):
         resident_step(events[k])
+    last = resident_step(events[-1])
     t_end.record()
     barrier()
     clocks = sampler.stop() if sampler else None
     launches = lib.pgica_kernel_launches() - launches0
     elapsed_ms = t_begin.elapsed_time(t_end)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    del last
     # order of marks: 0 start,1 after fwd_policy,2 after fwd_ref,3 after dpo,4 after dW (or the fused backward),
     # 5 after dH,(6 after all-reduce)
     names_in_order = ["fwd_policy", "fwd_reference", "dpo_scalar", "bwd_dH_dW" if fused else "bwd_dW", "bwd_dH"] + \
@@ -875,7 +901,13 @@ def main():
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -47,8 +47,10 @@ def test_every_entry_point_cites_the_reference():
 
 
 def test_library_is_sm100a_only(lib):
-    from preference_guided_image_captioning_alignment_b200 import _lib
-    out = subprocess.run(["cuobjdump", "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    from preference_guided_image_captioning_alignment_b200 import _build, _lib
+    # the cuobjdump of the toolkit that built the library: CUDA's bin directory need not be on PATH
+    cuobjdump = os.path.join(os.path.dirname(os.path.realpath(_build.nvcc_path())), "cuobjdump")
+    out = subprocess.run([cuobjdump, "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
 
