@@ -40,7 +40,6 @@ constexpr int kMaxEpiGroups = 2;
 constexpr int epi_groups(bool cols) { return cols ? 2 : 1; }
 constexpr int block_threads(bool cols) { return 128 + 128 * epi_groups(cols); }
 constexpr int kEpilogueWarp0 = 4;
-constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kLn2 = 0.6931471805599453f;
 
 struct GemmLseParams {

@@ -2,21 +2,59 @@
 // plumbing kernels (small.cu) on the caller's stream, carving the caller's workspace.  No allocation,
 // no synchronisation, no host round trip (the upstream gradient is read on the device).
 #include "common.h"
+#include "sgg_tile.cuh"
 
-extern "C" {
-
-using namespace pgica;
-}
 namespace pgica {
+size_t sggx_workspace_bytes();  // sgg_x.cu
 bool sggf_supported(int64_t mx, int64_t my, int64_t k);  // sgg_f.cu
 bool sggf_single_chunk(int64_t mx, int64_t my, int64_t k);
 size_t sggf_workspace_bytes();
-int sggf_dispatch(const void* x, const void* y, int64_t mx, int64_t my, int64_t k, float scale, const float* r_lse,
-                  const float* r_coef, const int32_t* r_tgt, const float* c_lse, const float* c_coef,
-                  const int32_t* c_tgt, void* out_x, int out_x_is_bf16, void* out_y, int out_y_is_bf16,
-                  void* workspace, size_t workspace_bytes, cudaStream_t st, uint32_t* progress,
-                  int64_t rows_per_segment, bool shared_exponential);
+int sggf_dispatch(const void* x, const void* y, int64_t mx, int64_t my, int64_t k, const SoftmaxGradStats& stats,
+                  void* out_x, int out_x_is_bf16, void* out_y, int out_y_is_bf16, void* workspace,
+                  size_t workspace_bytes, cudaStream_t st, uint32_t* progress, int64_t rows_per_segment,
+                  bool shared_exponential);
+
+namespace {
+// Exchange workspace of backward(): the one-product kernel's, or the dual kernel's when that takes the shape.
+size_t backward_workspace_bytes(int64_t mx, int64_t my, int64_t k) {
+  const size_t one = sggx_workspace_bytes();
+  return sggf_supported(mx, my, k) && sggf_workspace_bytes() > one ? sggf_workspace_bytes() : one;
+}
+
+// OutX = G Y (when out_x) and OutY = G^T X (when out_y).  Both from one recomputation of the logits (sgg_f.cu) when the
+// dual kernel takes the shape, the workspace holds its exchange ring and a bf16 OutY can be written in one chunk; else
+// one launch per product, OutY with the statistics of G^T.  `st` carries scale * log2(e); `scale` is the same scale
+// for the C entry points.  shared_exponential: one exponential per element for both terms (see sggf_kernel).
+int backward(const void* x, const void* y, int64_t mx, int64_t my, int64_t k, float scale, const SoftmaxGradStats& st,
+             void* out_x, int out_x_is_bf16, void* out_y, int out_y_is_bf16, void* ws, size_t ws_bytes, void* stream,
+             bool shared_exponential) {
+  if (out_x && out_y && sggf_supported(mx, my, k) && ws && ws_bytes >= sggf_workspace_bytes() &&
+      (!out_y_is_bf16 || sggf_single_chunk(mx, my, k))) {
+    if (shared_exponential)
+      return sggf_dispatch(x, y, mx, my, k, st, out_x, out_x_is_bf16, out_y, out_y_is_bf16, ws, ws_bytes,
+                           static_cast<cudaStream_t>(stream), nullptr, 0, true);
+    return pgica_softmax_grad_gemm_dual(x, y, mx, my, k, scale, st.r_lse, st.r_coef, st.r_tgt, st.c_lse, st.c_coef,
+                                        st.c_tgt, out_x, out_x_is_bf16, out_y, out_y_is_bf16, ws, ws_bytes, stream);
+  }
+  int rc;
+  if (out_x) {
+    rc = pgica_softmax_grad_gemm(x, y, mx, my, k, scale, st.r_lse, st.r_coef, st.r_tgt, st.c_lse, st.c_coef, st.c_tgt,
+                                 out_x, out_x_is_bf16, ws, ws_bytes, stream);
+    if (rc != PGICA_OK) return rc;
+  }
+  if (out_y) {
+    const SoftmaxGradStats t = st.transposed();
+    rc = pgica_softmax_grad_gemm(y, x, my, mx, k, scale, t.r_lse, t.r_coef, t.r_tgt, t.c_lse, t.c_coef, t.c_tgt, out_y,
+                                 out_y_is_bf16, ws, ws_bytes, stream);
+    if (rc != PGICA_OK) return rc;
+  }
+  return PGICA_OK;
+}
+}  // namespace
 }  // namespace pgica
+
+using namespace pgica;
+
 extern "C" {
 
 // ---- internal building blocks defined in the other translation units
@@ -28,11 +66,8 @@ int pgica_lmhead_logprob_workspace_bytes(int64_t nseq, int64_t seqlen, int64_t d
   int rc = pgica_gemm_lse_workspace_bytes(nseq * seqlen, vocab, d, &g);
   if (rc != PGICA_OK) return rc;
   // backward: one float per row for the coefficients + the G-tile exchange ring; forward: the LSE partials
-  size_t x = 0;
-  rc = pgica_softmax_grad_gemm_workspace_bytes(nseq * seqlen, vocab, d, &x);
-  if (rc != PGICA_OK) return rc;
-  if (sggf_supported(nseq * seqlen, vocab, d) && sggf_workspace_bytes() > x) x = sggf_workspace_bytes();
-  const size_t bwd = align_up((size_t)(nseq * seqlen) * sizeof(float), 256) + x;
+  const size_t bwd =
+      align_up((size_t)(nseq * seqlen) * sizeof(float), 256) + backward_workspace_bytes(nseq * seqlen, vocab, d);
   *bytes_host = g > bwd ? g : bwd;
   return PGICA_OK;
 }
@@ -62,24 +97,8 @@ int pgica_lmhead_rows_bwd(const void* hidden, const void* weight, const int32_t*
                           size_t workspace_bytes, void* stream) {
   PGICA_REQUIRE(hidden && weight && row_label && lse && ncoef, "lmhead_rows_bwd: null pointer");
   PGICA_REQUIRE(dhidden || dweight, "lmhead_rows_bwd: nothing to compute");
-  if (dhidden && dweight && sggf_supported(rows, vocab, d) && workspace && workspace_bytes >= sggf_workspace_bytes() &&
-      (!dweight_is_bf16 || sggf_single_chunk(rows, vocab, d)))
-    // both gradients from one recomputation of the logits (sgg_f.cu)
-    return pgica_softmax_grad_gemm_dual(hidden, weight, rows, vocab, d, 1.0f, lse, ncoef, row_label, nullptr, nullptr,
-                                        nullptr, dhidden, dhidden_is_bf16, dweight, dweight_is_bf16, workspace,
-                                        workspace_bytes, stream);
-  int rc;
-  if (dhidden) {
-    rc = pgica_softmax_grad_gemm(hidden, weight, rows, vocab, d, 1.0f, lse, ncoef, row_label, nullptr, nullptr,
-                                 nullptr, dhidden, dhidden_is_bf16, workspace, workspace_bytes, stream);
-    if (rc != PGICA_OK) return rc;
-  }
-  if (dweight) {
-    rc = pgica_softmax_grad_gemm(weight, hidden, vocab, rows, d, 1.0f, nullptr, nullptr, nullptr, lse, ncoef,
-                                 row_label, dweight, dweight_is_bf16, workspace, workspace_bytes, stream);
-    if (rc != PGICA_OK) return rc;
-  }
-  return PGICA_OK;
+  return backward(hidden, weight, rows, vocab, d, 1.0f, {kLog2e, lse, ncoef, row_label, nullptr, nullptr, nullptr},
+                  dhidden, dhidden_is_bf16, dweight, dweight_is_bf16, workspace, workspace_bytes, stream, false);
 }
 
 int pgica_lmhead_logprob_bwd(const void* hidden, const void* weight, const int32_t* row_label,
@@ -142,11 +161,8 @@ int pgica_ntxent_workspace_bytes(int64_t rows_a, int64_t rows_b, int64_t dim, si
   if (rc != PGICA_OK) return rc;
   size_t fwd = g1 > g2 ? g1 : g2;
   if (g3 > fwd) fwd = g3;
-  size_t x = 0;
-  rc = pgica_softmax_grad_gemm_workspace_bytes(rows_a, rows_b, dim, &x);
-  if (rc != PGICA_OK) return rc;
-  if (sggf_supported(rows_a, rows_b, dim) && sggf_workspace_bytes() > x) x = sggf_workspace_bytes();
-  const size_t bwd = 2 * align_up((size_t)rows_a * 4, 256) + 2 * align_up((size_t)rows_b * 4, 256) + x;
+  const size_t bwd = 2 * align_up((size_t)rows_a * 4, 256) + 2 * align_up((size_t)rows_b * 4, 256) +
+                     backward_workspace_bytes(rows_a, rows_b, dim);
   *bytes_host = fwd > bwd ? fwd : bwd;
   return PGICA_OK;
 }
@@ -169,7 +185,7 @@ int pgica_ntxent_fwd_bounded(const void* a, const void* b, int64_t rows_a, int64
                              int64_t diag_offset, float* lse_row, float* diag, float* lse_col_part, void* workspace,
                              size_t workspace_bytes, void* stream) {
   // bounded scheme: |t| <= inv_tau * log2(e) for unit-norm rows; keep 2 * that well inside the fp32 exponent range
-  if (!(inv_tau * 1.4426950408889634f * 2.0f < 100.0f))
+  if (!bounded_logits(inv_tau * kLog2e))
     return pgica_ntxent_fwd(a, b, rows_a, rows_b, dim, inv_tau, diag_offset, lse_row, diag, lse_col_part, workspace,
                             workspace_bytes, stream);
   PGICA_REQUIRE(a && b && lse_row && diag && lse_col_part, "ntxent_fwd_bounded: null pointer");
@@ -204,28 +220,10 @@ static int ntxent_bwd_impl(const void* a, const void* b, int64_t rows_a, int64_t
   if (rc != PGICA_OK) return rc;
   rc = pgica_ntxent_coef(grad_loss, grad_mult * inv_tau, rows_b, -diag_offset, rows_a, ccoef, ctgt, stream);
   if (rc != PGICA_OK) return rc;
-  if (da && db && sggf_supported(rows_a, rows_b, dim) && xws_bytes >= sggf_workspace_bytes() &&
-      (!db_is_bf16 || sggf_single_chunk(rows_a, rows_b, dim))) {
-    // dA and dB from one recomputation of the similarity tiles (sgg_f.cu).  Unit-norm rows: |logit| <= inv_tau, and the
-    // column targets built above mirror the row targets, so ONE exponential per element serves both softmax terms.
-    if (bounded)
-      return sggf_dispatch(a, b, rows_a, rows_b, dim, inv_tau, lse_row, rcoef, rtgt, lse_col, ccoef, ctgt, da,
-                           da_is_bf16, db, db_is_bf16, xws, xws_bytes, static_cast<cudaStream_t>(stream), nullptr, 0,
-                           true);
-    return pgica_softmax_grad_gemm_dual(a, b, rows_a, rows_b, dim, inv_tau, lse_row, rcoef, rtgt, lse_col, ccoef, ctgt,
-                                        da, da_is_bf16, db, db_is_bf16, xws, xws_bytes, stream);
-  }
-  if (da) {
-    rc = pgica_softmax_grad_gemm(a, b, rows_a, rows_b, dim, inv_tau, lse_row, rcoef, rtgt, lse_col, ccoef, ctgt, da,
-                                 da_is_bf16, xws, xws_bytes, stream);
-    if (rc != PGICA_OK) return rc;
-  }
-  if (db) {
-    rc = pgica_softmax_grad_gemm(b, a, rows_b, rows_a, dim, inv_tau, lse_col, ccoef, ctgt, lse_row, rcoef, rtgt, db,
-                                 db_is_bf16, xws, xws_bytes, stream);
-    if (rc != PGICA_OK) return rc;
-  }
-  return PGICA_OK;
+  // bounded: unit-norm rows, so |logit| <= inv_tau, and the column targets built above mirror the row targets: ONE
+  // exponential per element serves both softmax terms in the dual kernel
+  return backward(a, b, rows_a, rows_b, dim, inv_tau, {inv_tau * kLog2e, lse_row, rcoef, rtgt, lse_col, ccoef, ctgt}, da,
+                  da_is_bf16, db, db_is_bf16, xws, xws_bytes, stream, bounded);
 }
 
 int pgica_ntxent_bwd(const void* a, const void* b, int64_t rows_a, int64_t rows_b, int64_t dim, float inv_tau,
@@ -241,7 +239,7 @@ int pgica_ntxent_bwd_bounded(const void* a, const void* b, int64_t rows_a, int64
                              float grad_mult, void* da, int da_is_bf16, void* db, int db_is_bf16, void* workspace,
                              size_t workspace_bytes, void* stream) {
   // same bound as pgica_ntxent_fwd_bounded; a temperature too small for it takes the two-exponential form
-  const bool ok = inv_tau > 0.f && inv_tau * 1.4426950408889634f * 2.0f < 100.0f;
+  const bool ok = inv_tau > 0.f && bounded_logits(inv_tau * kLog2e);
   return ntxent_bwd_impl(a, b, rows_a, rows_b, dim, inv_tau, diag_offset, lse_row, lse_col, grad_loss, grad_mult, da,
                          da_is_bf16, db, db_is_bf16, workspace, workspace_bytes, stream, ok);
 }

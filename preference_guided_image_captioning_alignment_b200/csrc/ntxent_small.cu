@@ -13,7 +13,7 @@
 //            the operand rows re-streamed MN-major; results leave through shared memory as coalesced row stores.
 // The gradients are those of the loss itself (upstream gradient 1); autograd scales them by the upstream scalar.
 #include "common.h"
-#include "ptx.cuh"
+#include "sgg_tile.cuh"
 
 #include <mutex>
 
@@ -26,7 +26,6 @@ constexpr uint32_t kChunk = kT * kBK * 2;        // 16 KB: a [128][64] bf16 box
 constexpr int kRing = 4;                         // phase-1 stages of (A chunk + B chunk)
 constexpr int kPitch = kT + 1;                   // fp32 tile in shared memory, padded against bank conflicts
 constexpr int kThreads = 128;
-constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kLn2 = 0.6931471805599453f;
 // shared memory: [0, 128K) ring in phase 1, then {operand buffers 2 x 32K | G tile 32K | unused}; fp32 tile; vectors
 constexpr uint32_t kOffOp = 0, kOffG = 2 * 2 * kChunk, kOffZ = kRing * 2 * kChunk;
@@ -181,11 +180,7 @@ ntxent_small_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_const
         }
         gp[jj >> 1] = pack_bf16x2(g2[0], g2[1]);
       }
-      const uint32_t chunk_off = (ch >> 1) * kChunk;
-#pragma unroll
-      for (int c4 = 0; c4 < 4; ++c4)
-        st_smem_v4(g_local + chunk_off + sw128_offset(i, (ch & 1) * 4 + c4), gp[c4 * 4 + 0], gp[c4 * 4 + 1],
-                   gp[c4 * 4 + 2], gp[c4 * 4 + 3]);
+      store_g_chunk(g_local, i, ch, gp);
     }
     fence_proxy_async_smem();
   }

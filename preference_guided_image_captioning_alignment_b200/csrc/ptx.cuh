@@ -9,6 +9,8 @@
 
 namespace pgica {
 
+constexpr float kLog2e = 1.4426950408889634f;
+
 #ifndef PGICA_WATCHDOG_CYCLES
 // An mbarrier wait that has not completed after this many SM cycles (~2 s) traps instead of
 // hanging the GPU: a wrong phase/parity in a pipeline must fail loudly, not wedge the box.

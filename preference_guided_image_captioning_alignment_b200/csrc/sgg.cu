@@ -15,7 +15,7 @@
 #include <stdlib.h>
 
 #include "common.h"
-#include "ptx.cuh"
+#include "sgg_tile.cuh"
 
 namespace pgica {
 namespace {
@@ -29,19 +29,12 @@ constexpr uint32_t kChunkBytes = 128 * kBK * 2;   // 16 KB: a [128][64] bf16 box
 constexpr uint32_t kSlotBytes = 2 * kChunkBytes;  // 32 KB
 constexpr uint32_t kPBytes = kBM * kBT * 2;       // 32 KB
 constexpr int kThreads = 256;
-constexpr float kLog2e = 1.4426950408889634f;
 
 constexpr uint32_t kTmemOut = 0, kTmemZ = 256;  // column offsets: Out [0,256), Z0 [256,384), Z1 [384,512)
 
 struct SggParams {
   int mx, my, k, num_tiles, passes, ldo, out_bf16;
-  float c;  // scale * log2(e)
-  const float* r_lse;
-  const float* r_coef;
-  const int* r_tgt;
-  const float* c_lse;
-  const float* c_coef;
-  const int* c_tgt;
+  SoftmaxGradStats st;
   void* out;
 };
 
@@ -54,10 +47,8 @@ sgg_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUt
   uint8_t* smem = align_smem_1024(smem_raw);
   uint8_t* ring = smem;
   uint8_t* p_tile = smem + kSlots * kSlotBytes;
-  float* s_cl = reinterpret_cast<float*>(p_tile + kPBytes);
-  float* s_cc = s_cl + kBT;
-  int* s_ct = reinterpret_cast<int*>(s_cc + kBT);
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(s_ct + kBT);
+  float* s_col = reinterpret_cast<float*>(p_tile + kPBytes);
+  uint64_t* full_bar = reinterpret_cast<uint64_t*>(s_col + 3 * kBT);
   uint64_t* empty_bar = full_bar + kSlots;
   uint64_t* zfull_bar = empty_bar + kSlots;   // [2]
   uint64_t* zempty_bar = zfull_bar + 2;       // [2]
@@ -227,23 +218,12 @@ sgg_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUt
     const int row_in_blk = quarter * 32 + lane;
     const int row = m_blk * kBM + row_in_blk;
     const uint32_t lane_addr = static_cast<uint32_t>(quarter * 32) << 16;
-    float rl = 0.f, rc = 0.f;
-    int rt = -1;
-    if (kRow && row < p.mx) {
-      rl = p.r_lse[row] * kLog2e;
-      rc = p.r_coef[row];
-      rt = p.r_tgt ? p.r_tgt[row] : -1;
-    }
+    float rl, rc;
+    int rt;
+    load_row_stat<kRow>(p.st, row, row < p.mx, rl, rc, rt);
     auto load_col = [&](int j, float& l, float& cf, int& tg) {
       const int col = j * kBT + et;
-      l = 0.f;
-      cf = 0.f;
-      tg = -1;
-      if (kCol && col < p.my) {
-        l = p.c_lse[col] * kLog2e;
-        cf = p.c_coef[col];
-        tg = p.c_tgt ? p.c_tgt[col] : -1;
-      }
+      load_col_stat<kCol>(p.st, col, col < p.my, l, cf, tg);
     };
     float nl, nc;
     int nt;
@@ -253,9 +233,7 @@ sgg_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUt
     const uint32_t p_addr = smem_u32(p_tile);
     for (int j = 0; j < J; ++j) {
       if (kCol) {
-        s_cl[et] = nl;
-        s_cc[et] = nc;
-        s_ct[et] = nt;
+        stage_col_stat<false>(s_col, et, nl, nc, nt, p.st.c);
         asm volatile("bar.sync 1, 128;" ::: "memory");
         if (j + 1 < J) load_col(j + 1, nl, nc, nt);
       }
@@ -263,41 +241,17 @@ sgg_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUt
       tc_fence_after_sync();
       mbar_wait(pfree_bar, fphase ^ 1);  // MMA2(j-1) has finished reading the G tile
       fphase ^= 1;
-      const int col0 = j * kBT;
-      const int rrel = rt - col0;
+      const int rrel = rt - j * kBT;
 #pragma unroll 1
       for (int ch = 0; ch < kBT / 32; ++ch) {
         uint32_t r[32];
         tmem_ld_32x32(tmem_base + lane_addr + kTmemZ + zb * kBT + ch * 32, r);
         tmem_ld_wait();
         float g[32];
-#pragma unroll
-        for (int jj = 0; jj < 32; ++jj) {
-          const float t = __uint_as_float(r[jj]) * p.c;
-          float v = 0.f;
-          if (kRow) v = rc * fast_exp2(t - rl);
-          if (kCol) {
-            const int cj = ch * 32 + jj;
-            const float ccj = s_cc[cj];
-            v = fmaf(ccj, fast_exp2(t - s_cl[cj]), v);
-            if (s_ct[cj] == row) v -= ccj;
-          }
-          g[jj] = v;
-        }
-        if (kRow && rrel >= 0 && (rrel >> 5) == ch) {
-          const int jj0 = rrel & 31;
-#pragma unroll
-          for (int jj = 0; jj < 32; ++jj)
-            if (jj == jj0) g[jj] -= rc;
-        }
-        // 32 columns = 4 16-byte chunks of this row inside k-chunk (ch >> 1)
-        const uint32_t base = p_addr + (ch >> 1) * kChunkBytes;
-#pragma unroll
-        for (int c4 = 0; c4 < 4; ++c4) {
-          const uint32_t off = sw128_offset(row_in_blk, (ch & 1) * 4 + c4);
-          st_smem_v4(base + off, pack_bf16x2(g[c4 * 8 + 0], g[c4 * 8 + 1]), pack_bf16x2(g[c4 * 8 + 2], g[c4 * 8 + 3]),
-                     pack_bf16x2(g[c4 * 8 + 4], g[c4 * 8 + 5]), pack_bf16x2(g[c4 * 8 + 6], g[c4 * 8 + 7]));
-        }
+        g_chunk<kRow, kCol>(r, p.st.c, rl, rc, 0.f, row, rrel, s_col, ch, g);
+        uint32_t gp[16];
+        pack_g_chunk(g, gp);
+        store_g_chunk(p_addr, row_in_blk, ch, gp);
       }
       fence_proxy_async_smem();
       tc_fence_before_sync();
@@ -319,34 +273,7 @@ sgg_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUt
       tmem_ld_32x32(tmem_base + lane_addr + kTmemOut + ch * 32, r);
       tmem_ld_wait();
       const int col = ocol0 + ch * 32;
-      if (row < p.mx && col < p.k) {
-        if (col + 32 <= p.k) {
-          if (p.out_bf16) {
-            uint4* dst = reinterpret_cast<uint4*>(static_cast<__nv_bfloat16*>(p.out) + (size_t)row * p.ldo + col);
-#pragma unroll
-            for (int c4 = 0; c4 < 4; ++c4) {
-              uint4 v;
-              v.x = pack_bf16x2(__uint_as_float(r[c4 * 8 + 0]), __uint_as_float(r[c4 * 8 + 1]));
-              v.y = pack_bf16x2(__uint_as_float(r[c4 * 8 + 2]), __uint_as_float(r[c4 * 8 + 3]));
-              v.z = pack_bf16x2(__uint_as_float(r[c4 * 8 + 4]), __uint_as_float(r[c4 * 8 + 5]));
-              v.w = pack_bf16x2(__uint_as_float(r[c4 * 8 + 6]), __uint_as_float(r[c4 * 8 + 7]));
-              dst[c4] = v;
-            }
-          } else {
-            uint4* dst = reinterpret_cast<uint4*>(static_cast<float*>(p.out) + (size_t)row * p.ldo + col);
-#pragma unroll
-            for (int c4 = 0; c4 < 8; ++c4) dst[c4] = make_uint4(r[c4 * 4], r[c4 * 4 + 1], r[c4 * 4 + 2], r[c4 * 4 + 3]);
-          }
-        } else {
-          for (int jj = 0; jj < 32 && col + jj < p.k; ++jj) {
-            if (p.out_bf16)
-              static_cast<__nv_bfloat16*>(p.out)[(size_t)row * p.ldo + col + jj] =
-                  __float2bfloat16(__uint_as_float(r[jj]));
-            else
-              static_cast<float*>(p.out)[(size_t)row * p.ldo + col + jj] = __uint_as_float(r[jj]);
-          }
-        }
-      }
+      if (row < p.mx && col < p.k) store_out_chunk<true>(p.out, p.out_bf16, p.ldo, row, col, p.k, r);
     }
   }
 
@@ -357,10 +284,9 @@ sgg_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUt
 
 }  // namespace
 
-int sggx_dispatch(int cluster, const void* x, const void* y, int64_t mx, int64_t my, int64_t k, float scale,
-                  const float* r_lse, const float* r_coef, const int32_t* r_tgt, const float* c_lse,
-                  const float* c_coef, const int32_t* c_tgt, void* out, int out_is_bf16, void* workspace,
-                  size_t workspace_bytes, cudaStream_t st);
+int sggx_dispatch(int cluster, const void* x, const void* y, int64_t mx, int64_t my, int64_t k,
+                  const SoftmaxGradStats& stats, void* out, int out_is_bf16, void* workspace, size_t workspace_bytes,
+                  cudaStream_t st);
 size_t sggx_workspace_bytes();
 
 // Cluster size for the shared-recompute kernel (sgg_x.cu): the largest of {4, 2} whose 256-column slices tile k exactly,
@@ -399,10 +325,11 @@ extern "C" int pgica_softmax_grad_gemm(const void* x, const void* y, int64_t mx,
   PGICA_REQUIRE(!row || r_coef, "softmax_grad_gemm: r_coef missing");
   PGICA_REQUIRE(!col || c_coef, "softmax_grad_gemm: c_coef missing");
   PGICA_REQUIRE(scale > 0.f, "softmax_grad_gemm: scale must be positive");
+  const SoftmaxGradStats stats{scale * kLog2e, r_lse, r_coef, r_tgt, c_lse, c_coef, c_tgt};
   const int cluster = choose_cluster(k);
   if (cluster > 1 && workspace != nullptr && workspace_bytes > 0)
-    return sggx_dispatch(cluster, x, y, mx, my, k, scale, r_lse, r_coef, r_tgt, c_lse, c_coef, c_tgt, out, out_is_bf16,
-                         workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+    return sggx_dispatch(cluster, x, y, mx, my, k, stats, out, out_is_bf16, workspace, workspace_bytes,
+                         static_cast<cudaStream_t>(stream));
   SggParams p{};
   p.mx = (int)mx;
   p.my = (int)my;
@@ -411,13 +338,7 @@ extern "C" int pgica_softmax_grad_gemm(const void* x, const void* y, int64_t mx,
   p.passes = (int)ceil_div(k, kBD);
   p.ldo = (int)k;
   p.out_bf16 = out_is_bf16;
-  p.c = scale * kLog2e;
-  p.r_lse = r_lse;
-  p.r_coef = r_coef;
-  p.r_tgt = r_tgt;
-  p.c_lse = c_lse;
-  p.c_coef = c_coef;
-  p.c_tgt = c_tgt;
+  p.st = stats;
   p.out = out;
   CUtensorMap tm_x, tm_y;
   rc = make_tmap_bf16(&tm_x, x, mx, k, k, 128);
@@ -426,20 +347,13 @@ extern "C" int pgica_softmax_grad_gemm(const void* x, const void* y, int64_t mx,
   if (rc != PGICA_OK) return rc;
   const int64_t grid = ceil_div(mx, kBM) * p.passes;
   PGICA_REQUIRE(grid < (1ll << 31), "softmax_grad_gemm: grid too large");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-#define PGICA_LAUNCH_SGG(R, C)                                                                                    \
-  do {                                                                                                            \
-    PGICA_CUDA_OK(cudaFuncSetAttribute(sgg_kernel<R, C>, cudaFuncAttributeMaxDynamicSharedMemorySize,             \
-                                       (int)kSggSmem));                                                           \
-    sgg_kernel<R, C><<<(unsigned)grid, kThreads, kSggSmem, st>>>(tm_x, tm_y, p);                                   \
-  } while (0)
-  if (row && col)
-    PGICA_LAUNCH_SGG(true, true);
-  else if (row)
-    PGICA_LAUNCH_SGG(true, false);
-  else
-    PGICA_LAUNCH_SGG(false, true);
-#undef PGICA_LAUNCH_SGG
+  rc = with_terms(row, col, [&](auto r, auto c) {
+    auto kern = sgg_kernel<decltype(r)::value, decltype(c)::value>;
+    PGICA_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSggSmem));
+    kern<<<(unsigned)grid, kThreads, kSggSmem, static_cast<cudaStream_t>(stream)>>>(tm_x, tm_y, p);
+    return PGICA_OK;
+  });
+  if (rc != PGICA_OK) return rc;
   PGICA_CUDA_OK(cudaGetLastError());
   count_launches(1);
   return PGICA_OK;

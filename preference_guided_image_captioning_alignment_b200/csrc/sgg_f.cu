@@ -36,7 +36,7 @@
 #include <stdlib.h>
 
 #include "common.h"
-#include "ptx.cuh"
+#include "sgg_tile.cuh"
 
 #include <mutex>
 
@@ -63,7 +63,6 @@ constexpr int kStagesPerTile = kBT / 64;              // 2
 // the register file for the all-reduce kernel that runs beside it (peer_ar.cu); 384 threads would fill it.
 constexpr int epi_warps(bool row, bool col) { return col ? 8 : (void(row), 4); }
 constexpr int block_threads(bool row, bool col) { return 128 + 32 * epi_warps(row, col); }
-constexpr float kLog2e = 1.4426950408889634f;
 // No slack for aligning the dynamic window by hand: the array is declared __align__(1024) (checked on the device),
 // which keeps 1.5 KB of the SM's 228 KB free — enough for the 1 KB the hardware reserves per resident CTA, so that a
 // small shared-memory-free kernel (the progress-gated peer all-reduce, peer_ar.cu) can run BESIDE this one.
@@ -73,35 +72,6 @@ static_assert(2 * kPBytes + kCRing * kCStageBytes + kDrainBytes == 7 * 32768, "h
 
 #ifdef PGICA_TRACE
 __device__ long long* g_sggf_trace = nullptr;
-__device__ __forceinline__ long long ftrace_now() {
-#ifdef __CUDA_ARCH__
-  return clock64();
-#else
-  return 0;
-#endif
-}
-struct FLap {
-  long long t, acc[6];
-  __device__ FLap() : t(ftrace_now()) {
-    for (int i = 0; i < 6; ++i) acc[i] = 0;
-  }
-  __device__ void operator()(int i) {
-    const long long n = ftrace_now();
-    acc[i] += n - t;
-    t = n;
-  }
-  __device__ void flush(int base, int n) {
-    if (g_sggf_trace)
-      for (int i = 0; i < n; ++i) g_sggf_trace[(size_t)blockIdx.x * 24 + base + i] = acc[i];
-  }
-};
-#define LAP(i) lap(i)
-#define LAP_DECL FLap lap
-#define LAP_FLUSH(base, n) lap.flush(base, n)
-#else
-#define LAP(i) ((void)0)
-#define LAP_DECL ((void)0)
-#define LAP_FLUSH(base, n) ((void)0)
 #endif
 
 struct SggfParams {
@@ -114,13 +84,7 @@ struct SggfParams {
   int spread;             // 1: spread an X-holder's quads evenly over a pass (StepOffsets)
   int debug_producers_only;  // diagnostics: holders exit at once, producers publish nothing (results are garbage)
   int outx_bf16, outy_bf16;
-  float c;                // scale * log2(e)
-  const float* r_lse;
-  const float* r_coef;
-  const int* r_tgt;
-  const float* c_lse;
-  const float* c_coef;
-  const int* c_tgt;
+  SoftmaxGradStats st;
   void* out_x;
   void* out_y;
   uint32_t* progress;     // optional: progress[s] += 1 (release, gpu scope) whenever a drain warp's stores of a FINAL
@@ -373,10 +337,8 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
     if (threadIdx.x == 0) printf("pgica: sggf_kernel dynamic shared memory is not 1024-byte aligned\n");
     __trap();
   }
-  float* s_cl = reinterpret_cast<float*>(smem + 7 * 32768);
-  float* s_cc = s_cl + kBT;
-  int* s_ct = reinterpret_cast<int*>(s_cc + kBT);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(s_ct + kBT);
+  float* s_col = reinterpret_cast<float*>(smem + 7 * 32768);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(s_col + 3 * kBT);
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 32);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -442,7 +404,7 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
       int slot = 0;
       uint32_t phase = 0, stage_no = 0;
       const uint32_t lbar0 = mapa_u32(smem_u32(&full_bar[0]), 0);  // the leader's full barriers (shared::cluster)
-      LAP_DECL;
+      LAP_DECL(6);
       for_each_own_quad(p, pp, p.nP, [&](int q, int r0, int r, int c0, int c) {
         const int xrow = (2 * (r0 + r) + (int)rho) * kBM, yrow = (2 * (c0 + c) + (int)rho) * kBT;
         for (int kb = 0; kb < num_kb; ++kb, ++stage_no) {
@@ -466,14 +428,14 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
         }
       });
       LAP(0);
-      if (lane == 0 && warp == 0) LAP_FLUSH(4, 2);
+      if (lane == 0 && warp == 0) LAP_FLUSH(g_sggf_trace, 4, 2);
     } else if (warp == 1 && rho == 0) {
       // ---------------------------------------------------------------- MMA1 (leader): Z[256 x 256] = X[2rp, 2rp+1] Y[2cp, 2cp+1]^T
       constexpr uint32_t idesc1 = make_idesc_bf16(256, 256, 0, 0);
       const uint64_t desc_k = make_smem_desc(0, 16, 1024);
       int slot = 0;
       uint32_t phase = 0, n = 0;
-      LAP_DECL;
+      LAP_DECL(6);
       for_each_own_quad(p, pp, p.nP, [&](int q, int, int, int, int) {
         const uint32_t buf = n & 1u;
         LAP(0);
@@ -504,12 +466,12 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
         ++n;
       });
       LAP(0);
-      if (lane == 0) LAP_FLUSH(0, 3);
+      if (lane == 0) LAP_FLUSH(g_sggf_trace, 0, 3);
     } else if (warp == 3) {
       // ---------------------------------------------------------------- exchange: staging -> ring slot -> flag
       uint32_t n = 0, ntile = 0;
       const uint64_t pol_keep = l2_policy_evict_last();
-      LAP_DECL;
+      LAP_DECL(6);
       for_each_own_quad(p, pp, p.nP, [&](int q, int, int, int, int) {
         const uint32_t ds = n % (uint32_t)p.D, use = n / (uint32_t)p.D;
         for (int half = 0; half < 2; ++half) {
@@ -538,7 +500,7 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
         ++n;
       });
       LAP(0);
-      if (lane == 0) LAP_FLUSH(6, 4);
+      if (lane == 0) LAP_FLUSH(g_sggf_trace, 6, 4);
     } else if (warp >= 4) {
       // ---------------------------------------------------------------- epilogue: this CTA's Z rows -> two G tiles
       // Warp w reads the TMEM lanes of quarter w & 3 (the hardware's lane window of a warp) and, with eight warps, of
@@ -549,17 +511,13 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
       const uint32_t lane_addr = static_cast<uint32_t>(quarter * 32) << 16;
       const uint32_t g_local = smem_u32(staging);
       uint32_t n = 0, ntile = 0;
-      LAP_DECL;
+      LAP_DECL(6);
       for_each_own_quad(p, pp, p.nP, [&](int q, int r0, int r, int c0, int c) {
         const int row = (2 * (r0 + r) + (int)rho) * kBM + row_in_blk;
-        float rl = 0.f, rc = 0.f;
-        int rt = -1;
-        if (kRow && row < p.mx) {
-          rl = p.r_lse[row] * kLog2e;
-          rc = p.r_coef[row];
-          rt = p.r_tgt ? p.r_tgt[row] : -1;
-        }
-        const float rs = kShared ? rc * fast_exp2(p.c - rl) : 0.f;  // the row's factor of the shared exponential
+        float rl, rc;
+        int rt;
+        load_row_stat<kRow>(p.st, row, row < p.mx, rl, rc, rt);
+        const float rs = kShared ? rc * fast_exp2(p.st.c - rl) : 0.f;  // the row's factor of the shared exponential
         const uint32_t buf = n & 1u;
         LAP(0);
         mbar_wait(&zfull_bar[buf], (n >> 1) & 1u);
@@ -569,17 +527,10 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
           const int col0 = (2 * (c0 + c) + half) * kBT;
           if (kCol) {
             if (et < kBT) {
-              const int col = col0 + et;
-              float l = 0.f, cf = 0.f;
-              int tg = -1;
-              if (col < p.my) {
-                l = p.c_lse[col] * kLog2e;
-                cf = p.c_coef[col];
-                tg = p.c_tgt ? p.c_tgt[col] : -1;
-              }
-              s_cl[et] = kShared ? cf : l;                            // shared: the raw coefficient (one-hot fix-up)
-              s_cc[et] = kShared ? cf * fast_exp2(p.c - l) : cf;      //         the column's factor
-              s_ct[et] = tg;
+              float l, cf;
+              int tg;
+              load_col_stat<kCol>(p.st, col0 + et, col0 + et < p.my, l, cf, tg);
+              stage_col_stat<kShared>(s_col, et, l, cf, tg, p.st.c);
             }
             asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");
           }
@@ -592,32 +543,8 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
             tmem_ld_32x32(tmem_base + lane_addr + buf * 256u + half * kBT + ch * 32, rr);
             tmem_ld_wait();
             float g[32];
-#pragma unroll
-            for (int jj = 0; jj < 32; ++jj) {
-              if (kShared) {
-                g[jj] = fast_exp2(fmaf(__uint_as_float(rr[jj]), p.c, -p.c)) * (rs + s_cc[ch * 32 + jj]);
-                continue;
-              }
-              const float tz = __uint_as_float(rr[jj]) * p.c;
-              float v = 0.f;
-              if (kRow) v = rc * fast_exp2(tz - rl);
-              if (kCol) {
-                const int cj = ch * 32 + jj;
-                const float ccj = s_cc[cj];
-                v = fmaf(ccj, fast_exp2(tz - s_cl[cj]), v);
-                if (s_ct[cj] == row) v -= ccj;
-              }
-              g[jj] = v;
-            }
-            if (kRow && rrel >= 0 && (rrel >> 5) == ch) {
-              const int jj0 = rrel & 31;
-              const float hot = kShared ? rc + s_cl[ch * 32 + jj0] : rc;  // mirrored targets: both one-hots sit here
-#pragma unroll
-              for (int jj = 0; jj < 32; ++jj)
-                if (jj == jj0) g[jj] -= hot;
-            }
-#pragma unroll
-            for (int i = 0; i < 16; ++i) gp[cl * 16 + i] = pack_bf16x2(g[2 * i], g[2 * i + 1]);
+            g_chunk<kRow, kCol, kShared>(rr, p.st.c, rl, rc, rs, row, rrel, s_col, ch, g);
+            pack_g_chunk(g, gp + cl * 16);
           }
           if (half == 1) {
             tc_fence_before_sync();
@@ -627,15 +554,8 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
           mbar_wait(stfree_bar, (ntile & 1u) ^ 1u);  // the exchange warp's TMA store has read the previous tile
           LAP(3);
 #pragma unroll
-          for (int cl = 0; cl < kChunksPerWarp; ++cl) {
-            const int ch = wg * kChunksPerWarp + cl;
-#pragma unroll
-            for (int c4 = 0; c4 < 4; ++c4) {
-              const uint32_t off = (uint32_t)(ch >> 1) * kChunkBytes + sw128_offset(row_in_blk, (ch & 1) * 4 + c4);
-              st_smem_v4(g_local + off, gp[cl * 16 + c4 * 4 + 0], gp[cl * 16 + c4 * 4 + 1], gp[cl * 16 + c4 * 4 + 2],
-                         gp[cl * 16 + c4 * 4 + 3]);
-            }
-          }
+          for (int cl = 0; cl < kChunksPerWarp; ++cl)
+            store_g_chunk(g_local, row_in_blk, wg * kChunksPerWarp + cl, gp + cl * 16);
           fence_proxy_async_smem();
           mbar_arrive(stfull_bar);
           ++ntile;
@@ -645,7 +565,7 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
         ++n;
       });
       LAP(0);
-      if (et == 0) LAP_FLUSH(10, 5);
+      if (et == 0) LAP_FLUSH(g_sggf_trace, 10, 5);
     }
     tc_fence_before_sync();
     __syncthreads();
@@ -708,7 +628,7 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
     uint32_t n = 0;
     const uint64_t pol_keep = l2_policy_evict_last();
     const uint32_t gbar0 = mapa_u32(smem_u32(&gfull_bar[0]), 0);  // the leader's barriers (shared::cluster)
-    LAP_DECL;
+    LAP_DECL(6);
     for_each_holder_tile(
         p, is_y, hidx,
         [&](int q, int sel, int, int, bool, int) {
@@ -733,14 +653,14 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
         },
         [&](int, int, int) {});
     LAP(0);
-    if (lane == 0) LAP_FLUSH(4, 3);
+    if (lane == 0) LAP_FLUSH(g_sggf_trace, 4, 3);
   } else if (warp == 2) {
     // ------------------------------------------------------------------ TMA, operand rows: this CTA's half of X[r] / Y[c]
     // (independent of the producers: runs ahead of the G tiles by the depth of the ring)
     int slot = 0;
     uint32_t phase = 0;
     const uint32_t lbar0 = mapa_u32(smem_u32(&full_bar[0]), 0);
-    LAP_DECL;
+    LAP_DECL(6);
     for_each_holder_tile(
         p, is_y, hidx,
         [&](int, int sel, int rp, int cp, bool, int) {
@@ -768,7 +688,7 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
         [&](int, int, int) {});
     LAP(0);
 #ifdef PGICA_TRACE
-    if (lane == 0 && g_sggf_trace) g_sggf_trace[(size_t)blockIdx.x * 24 + 7] = lap.acc[3];
+    if (lane == 0 && g_sggf_trace) g_sggf_trace[(size_t)blockIdx.x * kTraceSlots + 7] = lap.acc[3];
 #endif
   } else if (warp == 1 && rho == 0) {
     // ------------------------------------------------------------------ MMA2 (leader): Out[256 x 512] += G(^T) * operand rows
@@ -778,7 +698,7 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
     const uint64_t desc_b = make_smem_desc(0, kBox64Bytes, 1024);      // operand rows, MN-major, 64-col boxes 8 KB apart
     int slot = 0;
     uint32_t phase = 0, n = 0;
-    LAP_DECL;
+    LAP_DECL(6);
     for_each_holder_tile(
         p, is_y, hidx,
         [&](int q, int sel, int, int, bool first, int period) {
@@ -836,7 +756,7 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
           __syncwarp();
         });
     LAP(0);
-    if (lane == 0) LAP_FLUSH(0, 4);
+    if (lane == 0) LAP_FLUSH(g_sggf_trace, 0, 4);
   } else if (warp >= 4 && warp < 8) {
     // ------------------------------------------------------------------ drain: accumulator -> OutX / OutY
     const int quarter = warp & 3;
@@ -852,7 +772,7 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
       asm volatile("fence.proxy.async.global;" ::: "memory");
       asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p.progress + seg), "r"(1u) : "memory");
     };
-    LAP_DECL;
+    LAP_DECL(6);
     for_each_holder_tile(
         p, is_y, hidx, [&](int, int, int, int, bool, int) {},
         [&](int period, int chunk, int pass) {
@@ -923,7 +843,7 @@ sggf_kernel(const __grid_constant__ CUtensorMap tm_x128, const __grid_constant__
       if (pending_seg >= 0) signal_progress(pending_seg);
     }
     __syncwarp();
-    if (threadIdx.x == 128) LAP_FLUSH(10, 3);
+    if (threadIdx.x == 128) LAP_FLUSH(g_sggf_trace, 10, 3);
   }
   tc_fence_before_sync();
   __syncthreads();
@@ -1240,11 +1160,10 @@ size_t sggf_workspace_bytes() {
   return nslots * (size_t)kPBytes + 2 * align_up(nslots * sizeof(uint32_t), 256);
 }
 
-int sggf_dispatch(const void* x, const void* y, int64_t mx, int64_t my, int64_t k, float scale, const float* r_lse,
-                  const float* r_coef, const int32_t* r_tgt, const float* c_lse, const float* c_coef,
-                  const int32_t* c_tgt, void* out_x, int out_x_is_bf16, void* out_y, int out_y_is_bf16,
-                  void* workspace, size_t workspace_bytes, cudaStream_t st, uint32_t* progress = nullptr,
-                  int64_t rows_per_segment = 0, bool shared_exponential = false) {
+int sggf_dispatch(const void* x, const void* y, int64_t mx, int64_t my, int64_t k, const SoftmaxGradStats& stats,
+                  void* out_x, int out_x_is_bf16, void* out_y, int out_y_is_bf16, void* workspace,
+                  size_t workspace_bytes, cudaStream_t st, uint32_t* progress = nullptr, int64_t rows_per_segment = 0,
+                  bool shared_exponential = false) {
   PGICA_REQUIRE(workspace != nullptr && (reinterpret_cast<uintptr_t>(workspace) & 255u) == 0,
                 "softmax_grad_gemm_dual: workspace missing or not 256-byte aligned");
   ProgressSpec sc;
@@ -1261,24 +1180,20 @@ int sggf_dispatch(const void* x, const void* y, int64_t mx, int64_t my, int64_t 
   p.S = (int)(k / kNC);
   p.outx_bf16 = out_x_is_bf16;
   p.outy_bf16 = out_y_is_bf16;
-  p.c = scale * kLog2e;
-  p.r_lse = r_lse;
-  p.r_coef = r_coef;
-  p.r_tgt = r_tgt;
-  p.c_lse = c_lse;
-  p.c_coef = c_coef;
-  p.c_tgt = c_tgt;
+  p.st = stats;
   p.out_x = out_x;
   p.out_y = out_y;
-  const bool row = r_lse != nullptr, col = c_lse != nullptr;
+  const bool row = stats.r_lse != nullptr, col = stats.c_lse != nullptr;
   if (shared_exponential) {
     // see sggf_kernel: |logit| <= scale, 2 scale log2(e) < 100, mirrored targets — promised by the caller (heads.cu)
-    PGICA_REQUIRE(row && col && r_tgt && c_tgt && 2.f * p.c < 100.f, "softmax_grad_gemm_dual: shared exponential misused");
+    PGICA_REQUIRE(row && col && stats.r_tgt && stats.c_tgt && bounded_logits(stats.c),
+                  "softmax_grad_gemm_dual: shared exponential misused");
     return plan_and_launch<true, true, true>(x, y, mx, my, k, p, workspace, workspace_bytes, sc, st);
   }
-  if (row && col) return plan_and_launch<true, true>(x, y, mx, my, k, p, workspace, workspace_bytes, sc, st);
-  if (row) return plan_and_launch<true, false>(x, y, mx, my, k, p, workspace, workspace_bytes, sc, st);
-  return plan_and_launch<false, true>(x, y, mx, my, k, p, workspace, workspace_bytes, sc, st);
+  return with_terms(row, col, [&](auto r, auto c) {
+    return plan_and_launch<decltype(r)::value, decltype(c)::value>(x, y, mx, my, k, p, workspace, workspace_bytes, sc,
+                                                                    st);
+  });
 }
 
 }  // namespace pgica
@@ -1322,27 +1237,40 @@ extern "C" int pgica_softmax_grad_gemm_dual_workspace_bytes(int64_t mx, int64_t 
   return PGICA_OK;
 }
 
+namespace {
+// Arguments both dual entry points take; `name` prefixes the error message.
+int check_dual_args(const char* name, const void* x, const void* y, int64_t mx, int64_t my, int64_t k, float scale,
+                    const float* r_lse, const float* r_coef, const float* c_lse, const float* c_coef, void* out_x,
+                    void* out_y) {
+  using namespace pgica;
+  int rc = pgica_device_check();
+  if (rc != PGICA_OK) return rc;
+  PGICA_REQUIRE(x && y && out_x && out_y, "%s: null operand", name);
+  PGICA_REQUIRE(mx > 0 && my > 0 && k > 0, "%s: bad shape (mx %lld my %lld k %lld)", name, (long long)mx, (long long)my,
+                (long long)k);
+  PGICA_REQUIRE(k % kNC == 0 && k / kNC <= 4, "%s: k must be 512, 1024, 1536 or 2048 (got %lld)", name, (long long)k);
+  PGICA_REQUIRE(mx < (1ll << 30) && my < (1ll << 30), "%s: dimension too large", name);
+  const bool row = r_lse != nullptr, col = c_lse != nullptr;
+  PGICA_REQUIRE(row || col, "%s: need row statistics, column statistics or both", name);
+  PGICA_REQUIRE(!row || r_coef, "%s: r_coef missing", name);
+  PGICA_REQUIRE(!col || c_coef, "%s: c_coef missing", name);
+  PGICA_REQUIRE(scale > 0.f, "%s: scale must be positive", name);
+  return PGICA_OK;
+}
+}  // namespace
+
 extern "C" int pgica_softmax_grad_gemm_dual(const void* x, const void* y, int64_t mx, int64_t my, int64_t k,
                                             float scale, const float* r_lse, const float* r_coef,
                                             const int32_t* r_tgt, const float* c_lse, const float* c_coef,
                                             const int32_t* c_tgt, void* out_x, int out_x_is_bf16, void* out_y,
                                             int out_y_is_bf16, void* workspace, size_t workspace_bytes, void* stream) {
   using namespace pgica;
-  int rc = pgica_device_check();
+  const int rc = check_dual_args("softmax_grad_gemm_dual", x, y, mx, my, k, scale, r_lse, r_coef, c_lse, c_coef, out_x,
+                                 out_y);
   if (rc != PGICA_OK) return rc;
-  PGICA_REQUIRE(x && y && out_x && out_y, "softmax_grad_gemm_dual: null operand");
-  PGICA_REQUIRE(mx > 0 && my > 0 && k > 0, "softmax_grad_gemm_dual: bad shape (mx %lld my %lld k %lld)", (long long)mx,
-                (long long)my, (long long)k);
-  PGICA_REQUIRE(k % kNC == 0 && k / kNC <= 4, "softmax_grad_gemm_dual: k must be 512, 1024, 1536 or 2048 (got %lld)",
-                (long long)k);
-  PGICA_REQUIRE(mx < (1ll << 30) && my < (1ll << 30), "softmax_grad_gemm_dual: dimension too large");
-  const bool row = r_lse != nullptr, col = c_lse != nullptr;
-  PGICA_REQUIRE(row || col, "softmax_grad_gemm_dual: need row statistics, column statistics or both");
-  PGICA_REQUIRE(!row || r_coef, "softmax_grad_gemm_dual: r_coef missing");
-  PGICA_REQUIRE(!col || c_coef, "softmax_grad_gemm_dual: c_coef missing");
-  PGICA_REQUIRE(scale > 0.f, "softmax_grad_gemm_dual: scale must be positive");
-  return sggf_dispatch(x, y, mx, my, k, scale, r_lse, r_coef, r_tgt, c_lse, c_coef, c_tgt, out_x, out_x_is_bf16, out_y,
-                       out_y_is_bf16, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+  return sggf_dispatch(x, y, mx, my, k, {scale * kLog2e, r_lse, r_coef, r_tgt, c_lse, c_coef, c_tgt}, out_x,
+                       out_x_is_bf16, out_y, out_y_is_bf16, workspace, workspace_bytes,
+                       static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int pgica_softmax_grad_gemm_dual_progress(const void* x, const void* y, int64_t mx, int64_t my, int64_t k,
@@ -1353,17 +1281,12 @@ extern "C" int pgica_softmax_grad_gemm_dual_progress(const void* x, const void* 
                                                      int32_t* increments_per_256_rows_host, void* workspace,
                                                      size_t workspace_bytes, void* stream) {
   using namespace pgica;
-  int rc = pgica_device_check();
+  const int rc = check_dual_args("softmax_grad_gemm_dual_progress", x, y, mx, my, k, scale, r_lse, r_coef, c_lse,
+                                 c_coef, out_x, out_y);
   if (rc != PGICA_OK) return rc;
-  PGICA_REQUIRE(x && y && out_x && out_y && progress, "softmax_grad_gemm_dual_progress: null operand");
-  PGICA_REQUIRE(mx > 0 && my > 0 && k > 0 && k % kNC == 0 && k / kNC <= 4,
-                "softmax_grad_gemm_dual_progress: bad shape (mx %lld my %lld k %lld)", (long long)mx, (long long)my,
-                (long long)k);
-  const bool row = r_lse != nullptr, col = c_lse != nullptr;
-  PGICA_REQUIRE(row || col, "softmax_grad_gemm_dual_progress: need row statistics, column statistics or both");
-  PGICA_REQUIRE((!row || r_coef) && (!col || c_coef) && scale > 0.f, "softmax_grad_gemm_dual_progress: bad statistics");
+  PGICA_REQUIRE(progress, "softmax_grad_gemm_dual_progress: null progress counters");
   if (increments_per_256_rows_host) *increments_per_256_rows_host = 8 * (int32_t)(k / kNC);  // 2 CTAs x S splits x 4 drain warps
-  return sggf_dispatch(x, y, mx, my, k, scale, r_lse, r_coef, r_tgt, c_lse, c_coef, c_tgt, out_x, out_x_is_bf16, out_y,
-                       out_y_is_bf16, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), progress,
-                       rows_per_segment);
+  return sggf_dispatch(x, y, mx, my, k, {scale * kLog2e, r_lse, r_coef, r_tgt, c_lse, c_coef, c_tgt}, out_x,
+                       out_x_is_bf16, out_y, out_y_is_bf16, workspace, workspace_bytes,
+                       static_cast<cudaStream_t>(stream), progress, rows_per_segment);
 }

@@ -20,7 +20,7 @@
 // (~20000 cycles); the epilogue + exchange need ~10000, and the slack costs no shared memory because finished tiles
 // wait in the exchange ring.
 #include "common.h"
-#include "ptx.cuh"
+#include "sgg_tile.cuh"
 
 #include <mutex>
 
@@ -40,52 +40,16 @@ constexpr uint32_t kStageBytes = kChunkBytes + 2 * kChunkBytes;  // 48 KB ring s
 constexpr int kRing = 4;
 constexpr int kXSlots = 16;  // exchange-ring depth in tiles (two rounds of a 4-CTA cluster)
 constexpr int kThreads = 256;
-constexpr float kLog2e = 1.4426950408889634f;
 constexpr uint32_t kTmemOut = 0, kTmemZ = 256;  // Out [0,256), Z [256,512) (single buffer, 256 columns)
 constexpr size_t kSmem = 1024 + kRing * kStageBytes + kPBytes + 3 * kBT * 4 + 512;
 
 #ifdef PGICA_TRACE
 __device__ long long* g_sggx_trace = nullptr;
-__device__ __forceinline__ long long xtrace_now() {
-#ifdef __CUDA_ARCH__
-  return clock64();
-#else
-  return 0;
-#endif
-}
-struct XLap {
-  long long t, acc[9];
-  __device__ XLap() : t(xtrace_now()) {
-    for (int i = 0; i < 9; ++i) acc[i] = 0;
-  }
-  __device__ void operator()(int i) {
-    const long long n = xtrace_now();
-    acc[i] += n - t;
-    t = n;
-  }
-  __device__ void flush(int base, int n) {
-    if (g_sggx_trace)
-      for (int i = 0; i < n; ++i) g_sggx_trace[(size_t)blockIdx.x * 24 + base + i] = acc[i];
-  }
-};
-#define LAP(i) lap(i)
-#define LAP_DECL XLap lap
-#define LAP_FLUSH(base, n) lap.flush(base, n)
-#else
-#define LAP(i) ((void)0)
-#define LAP_DECL ((void)0)
-#define LAP_FLUSH(base, n) ((void)0)
 #endif
 
 struct SggxParams {
   int mx, my, k, num_tiles, passes, num_items, ldo, out_bf16, prefetch_y;
-  float c;
-  const float* r_lse;
-  const float* r_coef;
-  const int* r_tgt;
-  const float* c_lse;
-  const float* c_coef;
-  const int* c_tgt;
+  SoftmaxGradStats st;
   void* out;
 };
 
@@ -113,10 +77,8 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
   uint8_t* smem = align_smem_1024(smem_raw);
   uint8_t* ring = smem;
   uint8_t* staging = smem + kRing * kStageBytes;  // this CTA's freshly produced G tile, source of the TMA store
-  float* s_cl = reinterpret_cast<float*>(staging + kPBytes);
-  float* s_cc = s_cl + kBT;
-  int* s_ct = reinterpret_cast<int*>(s_cc + kBT);
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(s_ct + kBT);
+  float* s_col = reinterpret_cast<float*>(staging + kPBytes);
+  uint64_t* full_bar = reinterpret_cast<uint64_t*>(s_col + 3 * kBT);
   uint64_t* empty_bar = full_bar + kRing;
   uint64_t* zfull_bar = empty_bar + kRing;   // [1] (+1 spare)
   uint64_t* zempty_bar = zfull_bar + 2;      // [1] (+1 spare)
@@ -186,7 +148,7 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
         phase ^= 1;
       }
     };
-    LAP_DECL;
+    LAP_DECL(9);
     for (int R = 0; R <= T; ++R) {
       {
         const int it = R / rounds, r = R - it * rounds;
@@ -264,7 +226,7 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
       }
     }
     LAP(0);
-    if (lane == 0) LAP_FLUSH(0, 4);
+    if (lane == 0) LAP_FLUSH(g_sggx_trace, 0, 4);
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer (whole warp, one elected lane)
     constexpr uint32_t idesc1 = make_idesc_bf16(kBM, kBT2, 0, 0);
@@ -282,7 +244,7 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
       }
     };
     uint32_t zuse = 0;  // own MMA1 tiles issued so far (Z is a single 256-column buffer)
-    LAP_DECL;
+    LAP_DECL(9);
     for (int R = 0; R <= T; ++R) {
       {
         const int own2 = (R % rounds) * C + (int)q;
@@ -367,14 +329,14 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
       }
     }
     LAP(0);
-    if (lane == 0) LAP_FLUSH(4, 5);
+    if (lane == 0) LAP_FLUSH(g_sggx_trace, 4, 5);
   } else if (warp == 3) {
     // ------------------------------------------------------------------ exchange warp
     // Takes each finished G tile from the staging buffer to the cluster: TMA store into the exchange ring, wait for
     // the store to complete, release it to every CTA.  Runs beside the epilogue warps, so the ~3000 cycles of store
     // completion + fences are off their critical path (they matter when k is small and the epilogue is the pace).
     uint32_t ntile = 0;
-    LAP_DECL;
+    LAP_DECL(9);
     for (int R = 0; R < T; ++R) {
       const int it = R / rounds, r = R - it * rounds;
       const int own2 = r * C + (int)q;
@@ -412,7 +374,7 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
       }
     }
     LAP(0);
-    if (lane == 0) LAP_FLUSH(18, 4);
+    if (lane == 0) LAP_FLUSH(g_sggx_trace, 18, 4);
   } else if (warp >= 4) {
     // ------------------------------------------------------------------ epilogue: Z -> G for this CTA's own tiles
     const int quarter = warp & 3;
@@ -421,7 +383,7 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
     const uint32_t lane_addr = static_cast<uint32_t>(quarter * 32) << 16;
     const uint32_t g_local = smem_u32(staging);
     uint32_t zuse = 0, ntile = 0;
-    LAP_DECL;
+    LAP_DECL(9);
     // Out slice of item number `itd` of this cluster: TMEM -> global, then hand TMEM back to the MMA warp
     auto drain_out = [&](int itd) {
       const int item_d = cluster_id + itd * num_clusters;
@@ -438,24 +400,7 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
         tmem_ld_32x32(tmem_base + lane_addr + kTmemOut + ch * 32, rr);
         tmem_ld_wait();
         const int col = ocol0 + ch * 32;
-        if (row_d < p.mx) {
-          if (p.out_bf16) {
-            uint4* dst = reinterpret_cast<uint4*>(static_cast<__nv_bfloat16*>(p.out) + (size_t)row_d * p.ldo + col);
-#pragma unroll
-            for (int c4 = 0; c4 < 4; ++c4) {
-              uint4 v;
-              v.x = pack_bf16x2(__uint_as_float(rr[c4 * 8 + 0]), __uint_as_float(rr[c4 * 8 + 1]));
-              v.y = pack_bf16x2(__uint_as_float(rr[c4 * 8 + 2]), __uint_as_float(rr[c4 * 8 + 3]));
-              v.z = pack_bf16x2(__uint_as_float(rr[c4 * 8 + 4]), __uint_as_float(rr[c4 * 8 + 5]));
-              v.w = pack_bf16x2(__uint_as_float(rr[c4 * 8 + 6]), __uint_as_float(rr[c4 * 8 + 7]));
-              dst[c4] = v;
-            }
-          } else {
-            uint4* dst = reinterpret_cast<uint4*>(static_cast<float*>(p.out) + (size_t)row_d * p.ldo + col);
-#pragma unroll
-            for (int c4 = 0; c4 < 8; ++c4) dst[c4] = make_uint4(rr[c4 * 4], rr[c4 * 4 + 1], rr[c4 * 4 + 2], rr[c4 * 4 + 3]);
-          }
-        }
+        if (row_d < p.mx) store_out_chunk<false>(p.out, p.out_bf16, p.ldo, row_d, col, p.k, rr);
       }
       tc_fence_before_sync();
       mbar_arrive(outfree_bar);
@@ -465,14 +410,7 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
     int rt = -1, nt = -1, gbase = 0;
     auto load_col = [&](int j, float& l, float& cf, int& tg) {
       const int col = j * kBT + et;
-      l = 0.f;
-      cf = 0.f;
-      tg = -1;
-      if (kCol && j < J && col < p.my) {
-        l = p.c_lse[col] * kLog2e;
-        cf = p.c_coef[col];
-        tg = p.c_tgt ? p.c_tgt[col] : -1;
-      }
+      load_col_stat<kCol>(p.st, col, j < J && col < p.my, l, cf, tg);
     };
     for (int R = 0; R < T; ++R) {
       const int it = R / rounds, r = R - it * rounds;
@@ -480,14 +418,7 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
         const int m_blk = (cluster_id + it * num_clusters) / p.passes;
         row = m_blk * kBM + row_in_blk;
         gbase = it * J;
-        rl = 0.f;
-        rc = 0.f;
-        rt = -1;
-        if (kRow && row < p.mx) {
-          rl = p.r_lse[row] * kLog2e;
-          rc = p.r_coef[row];
-          rt = p.r_tgt ? p.r_tgt[row] : -1;
-        }
+        load_row_stat<kRow>(p.st, row, row < p.mx, rl, rc, rt);
         load_col(2 * (int)q, nl, nc, nt);  // column statistics of the first G tile this CTA produces
       }
       {
@@ -504,14 +435,11 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
           if (t >= J) break;
           const bool last_half = (half == 1) || (t + 1 >= J);
           if (kCol) {
-            s_cl[et] = nl;
-            s_cc[et] = nc;
-            s_ct[et] = nt;
+            stage_col_stat<false>(s_col, et, nl, nc, nt, p.st.c);
             asm volatile("bar.sync 1, 128;" ::: "memory");
             load_col((half == 0 && t + 1 < J) ? t + 1 : 2 * (own2 + C), nl, nc, nt);  // next G tile of this CTA
           }
-          const int col0 = t * kBT;
-          const int rrel = rt - col0;
+          const int rrel = rt - t * kBT;
           uint32_t gp[kBT / 2];  // this thread's row of the G tile as bf16 pairs
 #pragma unroll
           for (int ch = 0; ch < kBT / 32; ++ch) {
@@ -519,27 +447,8 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
             tmem_ld_32x32(tmem_base + lane_addr + kTmemZ + half * kBT + ch * 32, rr);
             tmem_ld_wait();
             float g[32];
-#pragma unroll
-            for (int jj = 0; jj < 32; ++jj) {
-              const float tz = __uint_as_float(rr[jj]) * p.c;
-              float v = 0.f;
-              if (kRow) v = rc * fast_exp2(tz - rl);
-              if (kCol) {
-                const int cj = ch * 32 + jj;
-                const float ccj = s_cc[cj];
-                v = fmaf(ccj, fast_exp2(tz - s_cl[cj]), v);
-                if (s_ct[cj] == row) v -= ccj;
-              }
-              g[jj] = v;
-            }
-            if (kRow && rrel >= 0 && (rrel >> 5) == ch) {
-              const int jj0 = rrel & 31;
-#pragma unroll
-              for (int jj = 0; jj < 32; ++jj)
-                if (jj == jj0) g[jj] -= rc;
-            }
-#pragma unroll
-            for (int i = 0; i < 16; ++i) gp[ch * 16 + i] = pack_bf16x2(g[2 * i], g[2 * i + 1]);
+            g_chunk<kRow, kCol>(rr, p.st.c, rl, rc, 0.f, row, rrel, s_col, ch, g);
+            pack_g_chunk(g, gp + ch * 16);
           }
           if (last_half) {
             tc_fence_before_sync();
@@ -549,15 +458,7 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
           mbar_wait(stfree_bar, (ntile & 1u) ^ 1u);  // the exchange warp's TMA store has read the previous tile
           LAP(3);
 #pragma unroll
-          for (int ch = 0; ch < kBT / 32; ++ch) {
-            const uint32_t chunk_off = (ch >> 1) * kChunkBytes;
-#pragma unroll
-            for (int c4 = 0; c4 < 4; ++c4) {
-              const uint32_t off = chunk_off + sw128_offset(row_in_blk, (ch & 1) * 4 + c4);
-              st_smem_v4(g_local + off, gp[ch * 16 + c4 * 4 + 0], gp[ch * 16 + c4 * 4 + 1], gp[ch * 16 + c4 * 4 + 2],
-                         gp[ch * 16 + c4 * 4 + 3]);
-            }
-          }
+          for (int ch = 0; ch < kBT / 32; ++ch) store_g_chunk(g_local, row_in_blk, ch, gp + ch * 16);
           fence_proxy_async_smem();  // generic-proxy writes -> visible to the async proxy (the TMA store reads them)
           mbar_arrive(stfull_bar);   // hand the tile to the exchange warp
           ++ntile;
@@ -571,7 +472,7 @@ sggx_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CU
     }
     drain_out(n_my - 1);
     LAP(0);
-    if (et == 0) LAP_FLUSH(9, 9);
+    if (et == 0) LAP_FLUSH(g_sggx_trace, 9, 9);
   }
 
   tc_fence_before_sync();
@@ -660,10 +561,9 @@ extern "C" int pgica_debug_set_sggx_trace(void* buf) {
 size_t sggx_workspace_bytes() { return (size_t)64 * kXSlots * kPBytes; }
 
 // Called by pgica_softmax_grad_gemm when k is a multiple of 256*C.  Returns PGICA_OK or an error code.
-int sggx_dispatch(int cluster, const void* x, const void* y, int64_t mx, int64_t my, int64_t k, float scale,
-                  const float* r_lse, const float* r_coef, const int32_t* r_tgt, const float* c_lse,
-                  const float* c_coef, const int32_t* c_tgt, void* out, int out_is_bf16, void* workspace,
-                  size_t workspace_bytes, cudaStream_t st) {
+int sggx_dispatch(int cluster, const void* x, const void* y, int64_t mx, int64_t my, int64_t k,
+                  const SoftmaxGradStats& stats, void* out, int out_is_bf16, void* workspace, size_t workspace_bytes,
+                  cudaStream_t st) {
   PGICA_REQUIRE(workspace != nullptr && (reinterpret_cast<uintptr_t>(workspace) & 127u) == 0,
                 "softmax_grad_gemm: exchange workspace missing or not 128-byte aligned");
   SggxParams p{};
@@ -678,13 +578,7 @@ int sggx_dispatch(int cluster, const void* x, const void* y, int64_t mx, int64_t
   p.ldo = (int)k;
   p.out_bf16 = out_is_bf16;
   p.prefetch_y = (my * k * 2 > (int64_t)(32 << 20)) ? 1 : 0;  // only an operand that cannot sit in L2
-  p.c = scale * kLog2e;
-  p.r_lse = r_lse;
-  p.r_coef = r_coef;
-  p.r_tgt = r_tgt;
-  p.c_lse = c_lse;
-  p.c_coef = c_coef;
-  p.c_tgt = c_tgt;
+  p.st = stats;
   p.out = out;
   CUtensorMap tm_x, tm_y, tm_y32, tm_y96;
   int rc = make_tmap_bf16(&tm_x, x, mx, k, k, 128);
@@ -695,16 +589,12 @@ int sggx_dispatch(int cluster, const void* x, const void* y, int64_t mx, int64_t
   if (rc != PGICA_OK) return rc;
   rc = make_tmap_bf16(&tm_y96, y, my, k, k, 96);  // MMA2 operand, rows 32..127 (a slot of its own)
   if (rc != PGICA_OK) return rc;
-  const bool row = r_lse != nullptr, col = c_lse != nullptr;
-#define PGICA_SGGX(CC)                                                                                    \
-  do {                                                                                                    \
-    if (row && col) return launch<CC, true, true>(tm_x, tm_y, tm_y32, tm_y96, workspace, workspace_bytes, p, st);   \
-    if (row) return launch<CC, true, false>(tm_x, tm_y, tm_y32, tm_y96, workspace, workspace_bytes, p, st);         \
-    return launch<CC, false, true>(tm_x, tm_y, tm_y32, tm_y96, workspace, workspace_bytes, p, st);                  \
-  } while (0)
-  if (cluster == 2) PGICA_SGGX(2);
-  if (cluster == 4) PGICA_SGGX(4);
-#undef PGICA_SGGX
+  if (cluster == 2 || cluster == 4)
+    return with_terms(stats.r_lse != nullptr, stats.c_lse != nullptr, [&](auto r, auto c) {
+      constexpr bool kRow = decltype(r)::value, kCol = decltype(c)::value;
+      return cluster == 2 ? launch<2, kRow, kCol>(tm_x, tm_y, tm_y32, tm_y96, workspace, workspace_bytes, p, st)
+                          : launch<4, kRow, kCol>(tm_x, tm_y, tm_y32, tm_y96, workspace, workspace_bytes, p, st);
+    });
   set_error("softmax_grad_gemm: unsupported cluster size %d", cluster);
   return PGICA_ERR_INVALID_ARGUMENT;
 }

@@ -7,7 +7,6 @@
 namespace pgica {
 namespace {
 
-constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kLn2 = 0.6931471805599453f;
 
 __device__ __forceinline__ float load_mask(const void* mask, int kind, size_t i) {

@@ -14,15 +14,12 @@ sys.path.insert(0, ROOT)
 PKG = os.path.join(ROOT, "preference_guided_image_captioning_alignment_b200")
 TRACE_LIB = os.path.join(PKG, "libpgica_trace.so")
 
-# layout written by sgg_x.cu (exchange through L2); the DSMEM kernel (PGICA_SGG_EXCHANGE=dsmem) has its own layout
+# layout written by sgg_x.cu (exchange through L2)
 NAMES = ["prod_other", "prod_wait_empty_mma1", "prod_wait_empty_mma2", "prod_wait_gready",
          "mma_issue", "mma_wait_zempty_outfree", "mma_wait_full1", "mma_wait_gtile", "mma_wait_full2",
          "epi_other", "epi_wait_zfull", "epi_compute", "epi_wait_stfree", "epi_stage_write", "epi_wait_outfull",
          "epi_unused6", "epi_unused7", "epi_unused8",
          "xw_other", "xw_wait_stfull", "xw_wait_gdone", "xw_store_fence_arrive"]
-NAMES_DSMEM = ["prod_other", "prod_wait_empty_mma1", "prod_wait_empty_mma2",
-               "mma_issue", "mma_wait_zempty", "mma_wait_full1", "mma_wait_gfull", "mma_wait_full2",
-               "epi_other", "epi_wait_zfull", "epi_wait_gfree", "epi_compute", "epi_barsync"]
 
 
 def build():
@@ -39,10 +36,9 @@ def run():
     from preference_guided_image_captioning_alignment_b200 import _lib
     from preference_guided_image_captioning_alignment_b200 import functional as F
     lib = _lib.load()
-    dsmem = False  # the DSMEM-exchange kernel was retired in round 2
-    setter = lib.pgica_debug_set_sgg_trace if dsmem else lib.pgica_debug_set_sggx_trace
+    setter = lib.pgica_debug_set_sggx_trace
     setter.argtypes = [ctypes.c_void_p]
-    names = NAMES_DSMEM if dsmem else NAMES
+    names = NAMES
     dev = "cuda"
     torch.manual_seed(0)
     for mode, mx, my in (("row", 4064, 50257), ("col", 50257, 4064)):
@@ -54,7 +50,7 @@ def run():
         tgt = torch.randint(0, my if mode == "row" else mx, lse.shape, device=dev, dtype=torch.int32)
         st = (lse, coef, tgt)
         grid = ((mx + 127) // 128) * 4
-        buf = torch.zeros(max(grid, 1024), 16 if dsmem else 24, dtype=torch.int64, device=dev)
+        buf = torch.zeros(max(grid, 1024), 24, dtype=torch.int64, device=dev)
         kw = dict(row=st) if mode == "row" else dict(col=st)
         for _ in range(2):
             F.softmax_grad_gemm(x, y, 1.0, **kw)
@@ -68,7 +64,7 @@ def run():
         t = buf.cpu().double()
         t = t[t.sum(1) > 0]  # CTAs that ran (the persistent kernel launches fewer than `grid`)
         grid = t.shape[0]
-        tot_mma = t[:, 3:8].sum(1) if dsmem else t[:, 4:9].sum(1)
+        tot_mma = t[:, 4:9].sum(1)
         res = {"mode": mode, "grid": grid, "ms": e0.elapsed_time(e1),
                "mma_total_cycles_mean": tot_mma.mean().item(), "mma_total_cycles_max": tot_mma.max().item()}
         for i, n in enumerate(names):
