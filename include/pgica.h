@@ -395,6 +395,29 @@ int pgica_grad_norm_clip(const void* const* grads_host, const int64_t* numels_ho
                          size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * SURVEY 8(f) row 2, the optimizer step that follows the clip (pkg/training/trainer.py:494-520, 619-633:
+ * torch.optim.AdamW after clip_grad_norm_) — AdamW over ALL tensors of a parameter group in one launch, element for
+ * element torch/optim/adam.py::_single_tensor_adam with decoupled weight decay (s = the stored step):
+ *   p *= 1 - lr*wd;  m = lerp(m, g, 1 - beta1);  v = beta2*v + (1 - beta2)*g^2;
+ *   p -= (lr / bc1) * m / (sqrt(v) / sqrt(bc2) + eps),  bc1 = 1 - beta1^(s+1),  bc2 = 1 - beta2^(s+1)
+ * The per-tensor scalars are computed in double and rounded once to fp32; the arithmetic is fp32.
+ *   params_host[i], grads_host[i], exp_avgs_host[i], exp_avg_sqs_host[i]: device pointers of contiguous fp32 tensors of
+ *   numels_host[i] < 2^31 elements (any 4-byte alignment); steps_host[i]: device pointer of tensor i's fp32 step
+ *   counter, read by the update and incremented by a second launch after it.
+ *   grad_stats: NULL, or the 3 floats pgica_grad_norm_clip writes (clip = 0 computes them without touching the
+ *   gradients).  With grad_stats, a non-finite norm (grad_stats[2] == 0) writes nothing — no p, m, v or step — and a
+ *   finite one runs the update on g * grad_stats[1] (one fp32 multiply: bit for bit what clipping the gradients in
+ *   place first gives).  The gradients in memory are never written.
+ *   Two launches, no host synchronisation; the tensor table (one entry per tensor) is uploaded on every call.
+ * workspace: pgica_adamw_workspace_bytes() bytes.
+ * ---------------------------------------------------------------------------------------------- */
+int pgica_adamw_workspace_bytes(int n_tensors, size_t* bytes_host);
+int pgica_adamw_step(void* const* params_host, const void* const* grads_host, void* const* exp_avgs_host,
+                     void* const* exp_avg_sqs_host, float* const* steps_host, const int64_t* numels_host,
+                     int n_tensors, double lr, double beta1, double beta2, double eps, double weight_decay,
+                     const float* grad_stats, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * SURVEY 8(f) row 4 — the caption decoder's cross-attention over ONE key/value token (pkg/models/model.py:528-535,
  * 594-601: nn.MultiheadAttention(query = token embeddings, key = value = the projected image) followed by
  * attention_norm(text + attended)).  With a single key the softmax is identically 1, so

@@ -24,6 +24,7 @@ _SCALARS = {
     "int32_t": ctypes.c_int32,
     "uint32_t": ctypes.c_uint32,
     "float": ctypes.c_float,
+    "double": ctypes.c_double,
     "size_t": ctypes.c_size_t,
 }
 

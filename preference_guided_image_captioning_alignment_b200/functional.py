@@ -491,6 +491,41 @@ def grad_norm_clip(grads, max_norm, clip=True):
 _GRADCLIP_CACHE = {}
 
 
+def adamw_step(params, grads, exp_avgs, exp_avg_sqs, steps, lr, beta1, beta2, eps, weight_decay, grad_stats=None):
+    """One AdamW step (decoupled weight decay, torch's single-tensor arithmetic) over lists of contiguous fp32 tensors
+    of one device, in place, in two launches (pgica_adamw_step): p, exp_avg and exp_avg_sq updated, then every 0-dim
+    fp32 `steps[i]` incremented.  `grad_stats` (optional): the (3,) tensor of grad_norm_clip(..., clip=False); the
+    update then runs on g * grad_stats[1], and writes nothing at all when grad_stats[2] == 0 (non-finite norm)."""
+    n = len(params)
+    if n == 0:
+        return
+    if not (len(grads) == len(exp_avgs) == len(exp_avg_sqs) == len(steps) == n):
+        raise ValueError("adamw_step: params, grads, exp_avgs, exp_avg_sqs and steps must have the same length")
+    _need_cuda(*params, *grads, *exp_avgs, *exp_avg_sqs, *steps, grad_stats)
+    dev = params[0].device
+    for i in range(n):
+        p, quad = params[i], (params[i], grads[i], exp_avgs[i], exp_avg_sqs[i])
+        for t in quad:
+            if t.dtype != torch.float32 or not t.is_contiguous() or t.layout != torch.strided:
+                raise ValueError("adamw_step: tensor %d: params, grads and state must be contiguous fp32" % i)
+            if t.numel() != p.numel() or t.device != dev:
+                raise ValueError("adamw_step: tensor %d: numel or device differs from its parameter" % i)
+        if steps[i].dtype != torch.float32 or steps[i].numel() != 1 or steps[i].device != dev:
+            raise ValueError("adamw_step: tensor %d: step must be a one-element fp32 tensor on the parameter's device" % i)
+    if grad_stats is not None and (grad_stats.dtype != torch.float32 or grad_stats.numel() < 3
+                                   or not grad_stats.is_contiguous() or grad_stats.device != dev):
+        raise ValueError("adamw_step: grad_stats must be the (3,) fp32 output of grad_norm_clip on the same device")
+    lib = _lib.load()
+    ptrs = lambda ts: (ctypes.c_void_p * n)(*[t.data_ptr() for t in ts])
+    numels = (ctypes.c_int64 * n)(*[p.numel() for p in params])
+    need = ctypes.c_size_t(0)
+    _lib.check(lib.pgica_adamw_workspace_bytes(n, ctypes.byref(need)))
+    ws = _ws(need.value, dev)
+    _lib.check(lib.pgica_adamw_step(ptrs(params), ptrs(grads), ptrs(exp_avgs), ptrs(exp_avg_sqs), ptrs(steps), numels, n,
+                                    float(lr), float(beta1), float(beta2), float(eps), float(weight_decay),
+                                    _p(grad_stats), _p(ws), ws.numel(), _stream()))
+
+
 # ----------------------------------------------------------------------------------------- compacted Stage-2 head
 class CompactRows:
     """What the forward of the compacted head keeps for the backward (device tensors + host counts)."""
