@@ -21,6 +21,17 @@ def l2_normalize(x, eps=1e-12):
     return x / n, n
 
 
+def l2_normalize_bwd(x, g, eps=1e-12):
+    """Gradient of F.normalize(x, dim=-1) for the upstream gradient g: (g - u <u, g>) / ||x|| with u = x / ||x||.  A
+    row with ||x|| < eps was divided by the constant eps (torch's clamp_min passes no gradient to the norm below its
+    bound): g / eps, no projection."""
+    x = np.asarray(x, F64)
+    g = np.asarray(g, F64)
+    u, n = l2_normalize(x, eps)
+    proj = np.where(np.sqrt(np.sum(x * x, axis=-1, keepdims=True)) < eps, 0.0, np.sum(u * g, axis=-1, keepdims=True))
+    return (g - u * proj) / n
+
+
 def effective_temperature(temperature, clamp_tau, min_temp=0.1, max_temp=2.0):
     """torch.clamp(self.temperature, min_temp, max_temp) — pkg/models/components.py:78 (ctor :45-59).
     The trainer-facing loss (pkg/models/model.py:988) divides by the raw temperature."""
@@ -42,8 +53,8 @@ def ntxent(x, y, temperature, normalize=False, clamp_tau=False, reduction="mean"
     b, B = x.shape[0], y.shape[0]
     tau = effective_temperature(temperature, clamp_tau)
     if normalize:
-        a, nx = l2_normalize(x)
-        c, ny = l2_normalize(y)
+        a, _ = l2_normalize(x)
+        c, _ = l2_normalize(y)
     else:
         a, c = x, y
     S = a @ c.T / tau
@@ -64,8 +75,7 @@ def ntxent(x, y, temperature, normalize=False, clamp_tau=False, reduction="mean"
     da = dS @ c / tau
     dc = dS.T @ a / tau
     if normalize:
-        dx = (da - a * np.sum(a * da, axis=-1, keepdims=True)) / nx
-        dy = (dc - c * np.sum(c * dc, axis=-1, keepdims=True)) / ny
+        dx, dy = l2_normalize_bwd(x, da), l2_normalize_bwd(y, dc)
     else:
         dx, dy = da, dc
     return dict(loss=loss, lse_row=lse_r, lse_col=lse_c, dx=dx, dy=dy, sim=S)

@@ -235,6 +235,10 @@ __global__ void rownorm_fwd_kernel(const T* __restrict__ x, int rows, int dim, f
 // dx = (g - xh * <xh, g>) * inv_norm with xh = x * inv_norm recomputed in fp32.  g is fp32 or bf16, rows `g_pitch`
 // elements apart; with g_second >= 0 the upstream gradient is g[:, 0:dim] + g[:, g_second:g_second+dim] (the two
 // column blocks a softmax-gradient GEMM over split operands [hi|hi|lo] produces).
+// A row the forward clamped (||x|| < eps) was divided by the constant eps: like torch's F.normalize, whose clamp_min
+// passes no gradient to the norm, it gets dx = g * inv_norm without the projection.  The sum of squares is recomputed
+// in the forward's lane / warp order, so 1 / sqrtf(ss) equals the stored inv_norm bit for bit when the forward did not
+// clamp and exceeds it when it did (a NaN row compares false and keeps its NaN gradient).
 template <typename TX, typename TG>
 __global__ void rownorm_bwd_kernel(const TX* __restrict__ x, const float* __restrict__ inv_norm,
                                    const TG* __restrict__ g, int rows, int dim, int64_t g_pitch, int64_t g_second,
@@ -245,9 +249,15 @@ __global__ void rownorm_bwd_kernel(const TX* __restrict__ x, const float* __rest
   const float inv = inv_norm[r];
   const TG* gr = g + (size_t)r * g_pitch;
   auto gv = [&](int k) { return g_second >= 0 ? ldf(gr, (size_t)k) + ldf(gr, (size_t)(g_second + k)) : ldf(gr, (size_t)k); };
-  float dot = 0.f;
-  for (int k = lane; k < dim; k += 32) dot = fmaf(ldf(x, (size_t)r * dim + k) * inv, gv(k), dot);
+  float dot = 0.f, ss = 0.f;
+  for (int k = lane; k < dim; k += 32) {
+    const float v = ldf(x, (size_t)r * dim + k);
+    ss = fmaf(v, v, ss);
+    dot = fmaf(v * inv, gv(k), dot);
+  }
   dot = warp_sum(dot);
+  ss = warp_sum(ss);
+  if (1.f / sqrtf(ss) > inv) dot = 0.f;
   for (int k = lane; k < dim; k += 32) {
     const size_t i = (size_t)r * dim + k;
     dx[i] = (gv(k) - ldf(x, i) * inv * dot) * inv;
