@@ -218,6 +218,9 @@ __global__ void ln_l2norm_fwd_kernel(const float* __restrict__ z, const float* _
 }
 
 // Backward of both outputs: de_total = de + (dn - nh <nh, dn>) * inv  (nh = e * inv), then the LayerNorm backward.
+// A row with ||e|| < eps_norm gets de + dn * inv and no projection: F.normalize's clamp_min passes no gradient to the
+// norm there.  The sum of squares is recomputed in the forward's order (same lanes, same fmaf chain, same butterfly),
+// so 1 / sqrtf(ss) exceeds the stored inv exactly when the forward clamped.
 // dgamma / dbeta partials per block of 8 rows (summed by the caller: deterministic).
 __global__ void ln_l2norm_bwd_kernel(const float* __restrict__ z, const float* __restrict__ gamma,
                                      const float* __restrict__ beta, const float* __restrict__ stats,
@@ -233,13 +236,16 @@ __global__ void ln_l2norm_bwd_kernel(const float* __restrict__ z, const float* _
   if (r < rows) {
     const float mu = stats[3 * r], rs = stats[3 * r + 1], inv = stats[3 * r + 2];
     const float* zr = z + (size_t)r * D;
-    float dot = 0.f;
+    float dot = 0.f, ss = 0.f;
     if (dn)
       for (int k = lane; k < D; k += 32) {
         const float ev = (zr[k] - mu) * rs * gamma[k] + beta[k];
+        ss = fmaf(ev, ev, ss);
         dot = fmaf(ev * inv, dn[(size_t)r * D + k], dot);
       }
     dot = warp_sum(dot);
+    ss = warp_sum(ss);
+    if (1.f / sqrtf(ss) > inv) dot = 0.f;
     float s1 = 0.f, s2 = 0.f;
     for (int k = lane; k < D; k += 32) {
       const float xh = (zr[k] - mu) * rs;

@@ -645,12 +645,25 @@ def lmhead_compact_bwd(ctx, weight_bf16, grad_seqs, need_dhidden=True, need_dwei
 
 
 # ----------------------------------------------------------------------------------------- SURVEY 8(f) rows 3, 4
+def _need_f32(what, **tensors):
+    """The kernels read these buffers as contiguous fp32 of the given shapes: anything else would be misread (or read
+    past its end).  tensors: name -> (tensor or None, expected shape)."""
+    for name, (t, shape) in tensors.items():
+        if t is None:
+            continue
+        if t.dtype != torch.float32 or tuple(t.shape) != tuple(shape) or not t.is_contiguous():
+            raise _lib.PgicaError("%s: %s must be a contiguous float32 tensor of shape %s (got %s %s%s)" % (
+                what, name, tuple(shape), t.dtype, tuple(t.shape), "" if t.is_contiguous() else ", not contiguous"))
+
+
 def xattn_ln_fwd(x, u, w, out_bias, gamma, beta, eps):
     """y = LayerNorm(x + out_bias + sum_h w[..., h] * u[:, h]) (pgica_xattn_ln_fwd).  -> (y, mean, rstd)"""
-    _need_cuda(x, u, w, out_bias, gamma, beta)
-    lib = _lib.load()
     B, T, E = x.shape
     H = u.shape[1]
+    _need_f32("xattn_ln_fwd", x=(x, (B, T, E)), u=(u, (B, H, E)), w=(w, (B, T, H)), out_bias=(out_bias, (E,)),
+              gamma=(gamma, (E,)), beta=(beta, (E,)))
+    _need_cuda(x, u, w, out_bias, gamma, beta)
+    lib = _lib.load()
     y = torch.empty_like(x)
     mean = torch.empty(B * T, dtype=torch.float32, device=x.device)
     rstd = torch.empty(B * T, dtype=torch.float32, device=x.device)
@@ -661,9 +674,12 @@ def xattn_ln_fwd(x, u, w, out_bias, gamma, beta, eps):
 
 def xattn_ln_bwd(dy, x, u, w, out_bias, gamma, mean, rstd):
     """-> (dx, du, dgamma_part [B, E], dbeta_part [B, E], dpre_sum_part [B, E])"""
-    lib = _lib.load()
     B, T, E = x.shape
     H = u.shape[1]
+    _need_f32("xattn_ln_bwd", dy=(dy, (B, T, E)), x=(x, (B, T, E)), u=(u, (B, H, E)), w=(w, (B, T, H)),
+              out_bias=(out_bias, (E,)), gamma=(gamma, (E,)), mean=(mean, (B * T,)), rstd=(rstd, (B * T,)))
+    _need_cuda(dy, x, u, w, out_bias, gamma, mean, rstd)
+    lib = _lib.load()
     f32 = dict(dtype=torch.float32, device=x.device)
     dx = torch.empty_like(x)
     du = torch.empty(B, H, E, **f32)
@@ -675,9 +691,10 @@ def xattn_ln_bwd(dy, x, u, w, out_bias, gamma, mean, rstd):
 
 def ln_l2norm_fwd(z, gamma, beta, eps_ln, eps_norm):
     """e = LayerNorm(z), n = e / max(||e||, eps_norm) in one launch.  -> (e, n, stats [rows, 3])"""
+    rows, D = z.shape
+    _need_f32("ln_l2norm_fwd", z=(z, (rows, D)), gamma=(gamma, (D,)), beta=(beta, (D,)))
     _need_cuda(z, gamma, beta)
     lib = _lib.load()
-    rows, D = z.shape
     e, n = torch.empty_like(z), torch.empty_like(z)
     stats = torch.empty(rows, 3, dtype=torch.float32, device=z.device)
     _lib.check(lib.pgica_ln_l2norm_fwd(_p(z), _p(gamma), _p(beta), rows, D, float(eps_ln), float(eps_norm), _p(e), _p(n),
@@ -687,8 +704,11 @@ def ln_l2norm_fwd(z, gamma, beta, eps_ln, eps_norm):
 
 def ln_l2norm_bwd(z, gamma, beta, stats, de, dn):
     """-> (dz, dgamma_part [ceil(rows / 8), D], dbeta_part)"""
-    lib = _lib.load()
     rows, D = z.shape
+    _need_f32("ln_l2norm_bwd", z=(z, (rows, D)), gamma=(gamma, (D,)), beta=(beta, (D,)), stats=(stats, (rows, 3)),
+              de=(de, (rows, D)), dn=(dn, (rows, D)))
+    _need_cuda(z, gamma, beta, stats, de, dn)
+    lib = _lib.load()
     nb = (rows + 7) // 8
     dz = torch.empty_like(z)
     dg = torch.empty(nb, D, dtype=torch.float32, device=z.device)

@@ -64,6 +64,7 @@ def collapsed_cross_attention_ln(text: torch.Tensor, vision: torch.Tensor, mha: 
         u = (v @ wo.t()).unsqueeze(1)                                             # (B, 1, E): heads already summed
     else:
         u = torch.einsum("bhd,ehd->bhe", v.view(B, H, hd), wo.view(E, H, hd))     # (B, H, E): one slice per head
+        keep_weights = keep_weights.to(torch.float32)                             # a bool / fp16 / fp64 mask as well
     return _XAttnLN.apply(text.float(), u.float(), keep_weights, mha.out_proj.bias, norm.weight, norm.bias, norm.eps)
 
 
@@ -97,20 +98,29 @@ class PendingResidual:
 
 
 def _xattn_forward(self, query, key, value, key_padding_mask=None, need_weights=True, attn_mask=None, **kw):
+    E = self.embed_dim
+    dropout = self.training and self.dropout > 0.0
     ok = (self.batch_first and key is value and query.is_cuda and query.dim() == 3 and key.dim() == 3 and
           key.shape[1] == 1 and key_padding_mask is None and attn_mask is None and self._qkv_same_embed_dim and
-          self.bias_k is None and not self.add_zero_attn and query.dtype == torch.float32)
+          self.bias_k is None and not self.add_zero_attn and query.dtype == torch.float32 and
+          E % 4 == 0 and E <= 4096 and not (dropout and self.num_heads > 32))    # the kernel's limits
     if not ok:
         return type(self).forward(self, query, key, value, key_padding_mask=key_padding_mask, need_weights=need_weights,
                                   attn_mask=attn_mask, **kw)
     return CollapsedAttention(self, key, query.shape, query.device), None
 
 
+def _fusable_norm(norm):
+    """A LayerNorm the kernels can apply: an fp32 weight and bias over the last dimension."""
+    return (norm.weight is not None and norm.bias is not None and norm.weight.dtype == torch.float32 and
+            norm.bias.dtype == torch.float32 and len(norm.normalized_shape) == 1)
+
+
 def _norm_forward(self, inp):
-    if isinstance(inp, PendingResidual):
+    if isinstance(inp, PendingResidual) and _fusable_norm(self):
         att = inp.attended
         return collapsed_cross_attention_ln(inp.text, att.vision, att.mha, self)
-    if isinstance(inp, CollapsedAttention):
+    if isinstance(inp, (CollapsedAttention, PendingResidual)):
         inp = inp.materialize()
     return TF.layer_norm(inp, self.normalized_shape, self.weight, self.bias, self.eps)
 
@@ -156,6 +166,8 @@ class _LnL2Norm(torch.autograd.Function):
 def ln_l2norm(z: torch.Tensor, norm: nn.LayerNorm, eps_norm: float = 1e-12):
     """(LayerNorm(z), F.normalize(LayerNorm(z), dim=-1)) for (rows, D) inputs: the tail of the projection heads and
     the normalisation in front of the contrastive head (model.py:141, 343, 828-829), one launch each way."""
+    if z.shape[-1] > 2048:
+        raise ValueError(f"ln_l2norm: dim {z.shape[-1]} > 2048, the largest row its backward takes")
     return _LnL2Norm.apply(z, norm.weight, norm.bias, norm.eps, eps_norm)
 
 
@@ -170,9 +182,11 @@ class NormalizedCarrier(torch.Tensor):
             t = args[0]
             p = kwargs.get("p", args[1] if len(args) > 1 else 2.0)
             dim = kwargs.get("dim", args[2] if len(args) > 2 else 1)
+            eps = kwargs.get("eps", args[3] if len(args) > 3 else 1e-12)
+            out = kwargs.get("out", args[4] if len(args) > 4 else None)
             twin = getattr(t, "_pgica_normalized", None)
-            if twin is not None and float(p) == 2.0 and dim in (-1, t.dim() - 1) and \
-                    float(kwargs.get("eps", 1e-12)) == 1e-12:
+            if twin is not None and out is None and float(p) == 2.0 and dim in (-1, t.dim() - 1) and \
+                    float(eps) == 1e-12:
                 return twin
         from torch.utils._pytree import tree_map
         plain = lambda x: x.as_subclass(torch.Tensor) if isinstance(x, NormalizedCarrier) else x
@@ -181,7 +195,7 @@ class NormalizedCarrier(torch.Tensor):
 
 
 def _proj_norm_forward(self, z):
-    if not (z.is_cuda and z.dim() == 2 and z.dtype == torch.float32 and z.shape[-1] <= 1024):
+    if not (z.is_cuda and z.dim() == 2 and z.dtype == torch.float32 and z.shape[-1] <= 1024 and _fusable_norm(self)):
         return TF.layer_norm(z, self.normalized_shape, self.weight, self.bias, self.eps)
     e, n = ln_l2norm(z, self)
     out = e.as_subclass(NormalizedCarrier)
