@@ -266,6 +266,44 @@ int pgica_gather_u32(const void* src, const int32_t* index, int64_t n, void* dst
 int pgica_scatter_u32(const void* src, const int32_t* index, int64_t n, void* dst, int64_t dst_n, void* stream);
 int pgica_scatter_rows(const void* src, int src_is_bf16, const int32_t* index, int64_t n, int64_t d, void* dst,
                        int dst_is_bf16, int64_t dst_rows, void* stream);
+/* ------------------------------------------------------------------------------------------------
+ * Compacted rows with the row count kept on the DEVICE, so that a whole compacted step can be captured into a CUDA
+ * graph and replayed: the caller sizes every launch from a host-chosen `rows_launch` (e.g. the scored rows its
+ * host-side masks give, rounded up to 256); the exact count n is never read back.  Positions [n, rows_launch) are
+ * padding: zero hidden row, label -1, coefficient 0, which pgica_gemm_lse and pgica_lmhead_rows_bwd treat as absent
+ * (finite LSE, zero gradient).  Every gather / scatter writes its whole destination on every call, so no value of an
+ * earlier call survives.  None of these takes a host-side data-dependent size or copies between host and device, and
+ * none needs a workspace (the GEMM stages take theirs from the existing queries at rows_launch rows).  Pointers that
+ * are not device memory are refused.
+ *
+ * Sequence sets (e.g. policy chosen, policy rejected; nset <= PGICA_COMPACT_MAX_SETS, rows_host[s] > 0 rows each) share
+ * one concatenated row space: set s owns rows [sum_{q<s} rows_host[q], ... + rows_host[s]).  row_weight, label_in and
+ * slot span all of it.
+ *
+ *   pgica_compact_rows_dev      one launch over all sets: slot[r] = position of row r among the scored rows (row_weight
+ *                               != 0, NaN counts; ascending, set after set), -1 if not scored; index[p] = r for p <
+ *                               min(n, rows_launch), -1 on [n, rows_launch); info int32[2 * nset + 2] = {counts[nset],
+ *                               offsets[nset], n, overflow}.  overflow = 1 when n > rows_launch: the rows that do not
+ *                               fit are dropped (never written out of bounds) and the scatters below mark them.
+ *   pgica_gather_rows_bf16_dev  dst[p][:] = bf16(row index[p] of its set's src_host[s] (fp32, or bf16 when
+ *                               src_is_bf16_host[s])), label_out[p] = label_in[index[p]]; zero row and label -1 at
+ *                               padding positions.  p in [0, rows_launch); d % 8 == 0.
+ *   pgica_gather_u32_dev        dst[p] = src[index[p]] for index[p] in [0, src_n), else 0; p in [0, n).
+ *   pgica_scatter_u32_dev       dst[r] = src[slot[r]] for slot[r] in [0, src_n), 0 for an unscored row, a quiet NaN for
+ *                               a scored row beyond src_n (overflow: its sequence and the loss become NaN); r in [0, rows).
+ *   pgica_scatter_rows_dev      dst[r][:] = src[slot[r]][:] (dtype change as asked) for slot[r] in [0, src_n), else
+ *                               zeros; r in [0, rows), d % 4 == 0.
+ * ---------------------------------------------------------------------------------------------- */
+#define PGICA_COMPACT_MAX_SETS 8
+int pgica_compact_rows_dev(const float* row_weight, int nset, const int64_t* rows_host, int64_t rows_launch,
+                           int32_t* index, int32_t* slot, int32_t* info, void* stream);
+int pgica_gather_rows_bf16_dev(int nset, const void* const* src_host, const int32_t* src_is_bf16_host,
+                               const int64_t* rows_host, const int32_t* index, int64_t rows_launch, int64_t d,
+                               void* dst_bf16, const int32_t* label_in, int32_t* label_out, void* stream);
+int pgica_gather_u32_dev(const void* src, int64_t src_n, const int32_t* index, int64_t n, void* dst, void* stream);
+int pgica_scatter_u32_dev(const void* src, int64_t src_n, const int32_t* slot, int64_t rows, void* dst, void* stream);
+int pgica_scatter_rows_dev(const void* src, int src_is_bf16, int64_t src_n, const int32_t* slot, int64_t rows,
+                           int64_t d, void* dst, int dst_is_bf16, void* stream);
 int pgica_lmhead_rows_workspace_bytes(int64_t rows, int64_t d, int64_t vocab, size_t* bytes_host);
 int pgica_lmhead_rows_bwd(const void* hidden, const void* weight, const int32_t* row_label, const float* lse,
                           const float* ncoef, int64_t rows, int64_t d, int64_t vocab, void* dhidden,

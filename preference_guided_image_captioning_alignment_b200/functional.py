@@ -644,6 +644,144 @@ def lmhead_compact_bwd(ctx, weight_bf16, grad_seqs, need_dhidden=True, need_dwei
     return dhs, dw
 
 
+class CompactRowsBucketed:
+    """What lmhead_compact_fwd_bucketed keeps for the backward.  All device tensors; nothing depends on the row count."""
+    __slots__ = ("hidden_c", "label_c", "lse_c", "index", "slot", "info", "row_weight", "shapes", "rows_launch",
+                 "length_normalize", "lse", "ztgt", "ref_lse", "ref_ztgt")
+
+
+def _row_sets(shapes):
+    rows = [nseq * T for nseq, T in shapes]
+    return len(rows), (ctypes.c_int64 * len(rows))(*rows), [sum(rows[:s]) for s in range(len(rows) + 1)]
+
+
+def _gather_bucketed(lib, srcs, rows_host, index, rows_launch, d, dev, label_in=None, label_out=None):
+    nset = len(srcs)
+    out = torch.empty(rows_launch, d, dtype=torch.bfloat16, device=dev)
+    ptrs = (ctypes.c_void_p * nset)(*[h.data_ptr() for h in srcs])
+    bf16 = (ctypes.c_int32 * nset)(*[1 if h.dtype == torch.bfloat16 else 0 for h in srcs])
+    _lib.check(lib.pgica_gather_rows_bf16_dev(nset, ptrs, bf16, rows_host, _p(index), rows_launch, d, _p(out),
+                                              _p(label_in), _p(label_out), _stream()))
+    return out
+
+
+def _hidden_sets(hiddens, d, what):
+    out = []
+    for h in hiddens:
+        if h.dim() != 3 or h.shape[-1] != d:
+            raise ValueError("%s: hidden (nseq, T, d) expected" % what)
+        out.append((h if h.dtype in (torch.float32, torch.bfloat16) else h.float()).contiguous())
+    return out
+
+
+def lmhead_compact_fwd_bucketed(hiddens, weight_bf16, labels, masks, rows_launch, length_normalize=False,
+                                ref_hiddens=None, ref_weight_bf16=None):
+    """lmhead_compact_fwd with the row count kept on the device: every launch is sized by `rows_launch` (>= the scored
+    rows of all sets; positions past them are padding that adds nothing), nothing is read back, so the call can be
+    captured into a CUDA graph.  With ref_hiddens / ref_weight_bf16 the frozen reference's log-probs come from the same
+    compacted index (no gradient).  More scored rows than rows_launch set info[-1] (overflow) and make the affected
+    sequences NaN.  -> ([seq_logp_s], [ref_seq_logp_s] or None, CompactRowsBucketed)"""
+    _need_cuda(weight_bf16, ref_weight_bf16, *hiddens, *labels, *[m for m in masks if m is not None],
+               *(ref_hiddens or []))
+    lib = _lib.load()
+    dev = weight_bf16.device
+    V, d = weight_bf16.shape
+    rows_launch = int(rows_launch)
+    srcs = _hidden_sets(hiddens, d, "lmhead_compact_fwd_bucketed")
+    shapes = [tuple(h.shape[:2]) for h in srcs]
+    nset, rows_host, begin = _row_sets(shapes)
+    R = begin[-1]
+    f32 = dict(dtype=torch.float32, device=dev)
+    ctx = CompactRowsBucketed()
+    ctx.shapes, ctx.rows_launch, ctx.length_normalize = shapes, rows_launch, bool(length_normalize)
+    row_label = torch.empty(R, dtype=torch.int32, device=dev)
+    ctx.row_weight = torch.empty(R, **f32)
+    for s in range(nset):
+        nseq, T = shapes[s]
+        kind, mask_c = mask_kind(masks[s])
+        lab = labels[s].contiguous() if labels[s].dtype == torch.int64 else labels[s].long().contiguous()
+        _lib.check(lib.pgica_prep_rows(_p(lab), _p(mask_c), kind, nseq, T, V, _p(row_label[begin[s]:]),
+                                       _p(ctx.row_weight[begin[s]:]), _stream()))
+    ctx.index = torch.empty(rows_launch, dtype=torch.int32, device=dev)
+    ctx.slot = torch.empty(R, dtype=torch.int32, device=dev)
+    ctx.info = torch.empty(2 * nset + 2, dtype=torch.int32, device=dev)
+    _lib.check(lib.pgica_compact_rows_dev(_p(ctx.row_weight), nset, rows_host, rows_launch, _p(ctx.index),
+                                          _p(ctx.slot), _p(ctx.info), _stream()))
+    ctx.label_c = torch.empty(rows_launch, dtype=torch.int32, device=dev)
+    ctx.hidden_c = _gather_bucketed(lib, srcs, rows_host, ctx.index, rows_launch, d, dev, row_label, ctx.label_c)
+
+    def seq_logprobs(hidden_c, weight):
+        lse_c, ztgt_c = gemm_lse(hidden_c, weight, 1.0, ctx.label_c)
+        lse, ztgt = torch.empty(R, **f32), torch.empty(R, **f32)
+        for src, dst in ((lse_c, lse), (ztgt_c, ztgt)):
+            _lib.check(lib.pgica_scatter_u32_dev(_p(src), rows_launch, _p(ctx.slot), R, _p(dst), _stream()))
+        seqs = [seq_reduce(lse[begin[s]:begin[s + 1]], ztgt[begin[s]:begin[s + 1]],
+                           ctx.row_weight[begin[s]:begin[s + 1]], *shapes[s], length_normalize) for s in range(nset)]
+        return seqs, lse_c, lse, ztgt
+
+    seqs, ctx.lse_c, ctx.lse, ctx.ztgt = seq_logprobs(ctx.hidden_c, weight_bf16)
+    ref_seqs = ctx.ref_lse = ctx.ref_ztgt = None
+    if ref_weight_bf16 is not None:
+        refs = _hidden_sets(ref_hiddens, d, "lmhead_compact_fwd_bucketed")
+        if [tuple(h.shape[:2]) for h in refs] != shapes:
+            raise ValueError("lmhead_compact_fwd_bucketed: reference hidden sets must have the policy's shapes")
+        ref_c = _gather_bucketed(lib, refs, rows_host, ctx.index, rows_launch, d, dev)
+        ref_seqs, _, ctx.ref_lse, ctx.ref_ztgt = seq_logprobs(ref_c, ref_weight_bf16)
+    return seqs, ref_seqs, ctx
+
+
+def lmhead_compact_bwd_bucketed(ctx, weight_bf16, grad_seqs, dhidden_outs=None, dweight_out=None,
+                                dhidden_dtypes=None, dweight_dtype=torch.float32):
+    """Backward of lmhead_compact_fwd_bucketed: one dual-kernel launch over the rows_launch compacted rows (padding rows
+    have coefficient 0).  dhidden_outs[s] / dweight_out: caller-owned destinations (written in full; dhidden is zero at
+    unscored rows), else allocated.  -> ([dhidden_s] (B_s, T_s, d), dweight (V, d))"""
+    _need_cuda(weight_bf16, *grad_seqs, dweight_out, *(dhidden_outs or []))
+    lib = _lib.load()
+    dev = weight_bf16.device
+    V, d = weight_bf16.shape
+    nset, _, begin = _row_sets(ctx.shapes)
+    R, n = begin[-1], ctx.rows_launch
+    coef = torch.empty(R, dtype=torch.float32, device=dev)
+    for s in range(nset):
+        nseq, T = ctx.shapes[s]
+        _lib.check(lib.pgica_row_coef(_p(grad_seqs[s].contiguous().float()), _p(ctx.row_weight[begin[s]:]), nseq, T,
+                                      1 if ctx.length_normalize else 0, -1.0, _p(coef[begin[s]:]), _stream()))
+    ncoef_c = torch.empty(n, dtype=torch.float32, device=dev)
+    _lib.check(lib.pgica_gather_u32_dev(_p(coef), R, _p(ctx.index), n, _p(ncoef_c), _stream()))
+    if dhidden_outs is not None:
+        dhidden_dtypes = [t.dtype for t in dhidden_outs]
+    dhidden_dtypes = dhidden_dtypes or [torch.float32] * nset
+    dhc_dtype = torch.bfloat16 if all(dt == torch.bfloat16 for dt in dhidden_dtypes) else torch.float32
+    dhc = torch.empty(n, d, dtype=dhc_dtype, device=dev)
+    if dweight_out is not None:
+        if tuple(dweight_out.shape) != (V, d) or not dweight_out.is_contiguous():
+            raise ValueError("dweight_out must be a contiguous (V, d) tensor")
+        dw = dweight_out
+    else:
+        dw = torch.empty(V, d, dtype=dweight_dtype, device=dev)
+    need = ctypes.c_size_t(0)
+    _lib.check(lib.pgica_lmhead_rows_workspace_bytes(n, d, V, ctypes.byref(need)))
+    ws = _ws(need.value, dev)
+    _lib.check(lib.pgica_lmhead_rows_bwd(_p(ctx.hidden_c), _p(weight_bf16), _p(ctx.label_c), _p(ctx.lse_c),
+                                         _p(ncoef_c), n, d, V, _p(dhc), 1 if dhc_dtype == torch.bfloat16 else 0,
+                                         _p(dw), 1 if dw.dtype == torch.bfloat16 else 0, _p(ws), ws.numel(),
+                                         _stream()))
+    dhs = []
+    for s in range(nset):
+        nseq, T = ctx.shapes[s]
+        if dhidden_outs is not None:
+            dh = dhidden_outs[s]
+            if tuple(dh.shape) != (nseq, T, d) or not dh.is_contiguous():
+                raise ValueError("dhidden_outs[%d] must be a contiguous (%d, %d, %d) tensor" % (s, nseq, T, d))
+        else:
+            dh = torch.empty(nseq, T, d, dtype=dhidden_dtypes[s], device=dev)
+        _lib.check(lib.pgica_scatter_rows_dev(_p(dhc), 1 if dhc_dtype == torch.bfloat16 else 0, n,
+                                              _p(ctx.slot[begin[s]:]), nseq * T, d, _p(dh),
+                                              1 if dh.dtype == torch.bfloat16 else 0, _stream()))
+        dhs.append(dh)
+    return dhs, dw
+
+
 # ----------------------------------------------------------------------------------------- SURVEY 8(f) rows 3, 4
 def _need_f32(what, **tensors):
     """The kernels read these buffers as contiguous fp32 of the given shapes: anything else would be misread (or read
@@ -742,6 +880,7 @@ def _device_guard(fn):
 
 for _name, _fn in list(globals().items()):
     if callable(_fn) and getattr(_fn, "__module__", None) == __name__ and not _name.startswith("_") \
-            and _name not in ("mask_kind", "ntxent_small_supported", "CompactRows"):
+            and _name not in ("mask_kind", "ntxent_small_supported", "CompactRows",
+                                                                     "CompactRowsBucketed"):
         globals()[_name] = _device_guard(_fn)
 del _name, _fn
