@@ -99,6 +99,23 @@ int pgica_gemm_lse_rowcol(const void* a, const void* b, int64_t rows, int64_t co
 int pgica_similarity(const void* a, const void* b, int64_t rows, int64_t cols, int64_t k, float scale, float* sim,
                      float* lse, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Retrieval ranks in both directions without the dense score matrix (image-text recall@K evaluation).
+ * S[i][j] = <a_i, b_j> in fp32 from the same tcgen05 tiles as pgica_similarity (rows = images, cols = captions).
+ * Caption j belongs to image owner(j) = col_owner[j]; col_owner == NULL pairs caption j with image j for j < rows.
+ * An owner outside [0, rows) means "no image": that caption gets rank -1 and touches nothing.
+ *   p_i         = max of S[i][j] over the captions j of image i (NaN if any of them is NaN)
+ *   row_rank[i] = #{j : S[i][j] > p_i},  -1 if image i owns no caption
+ *   col_rank[j] = #{i : S[i][j] > S[owner(j)][j]},  -1 if caption j has no owner
+ * Strict fp32 '>': ties count for the positive, a NaN threshold counts 0.  Two passes over the tiles: the tiles that
+ * hold a positive (p, q), then every tile (int32 counts, red.global.add: deterministic).  Four launches whatever the
+ * size, no host synchronisation.  a, b: bf16 [rows][k], [cols][k], k % 8 == 0.  row_rank: int32 [rows], col_rank:
+ * int32 [cols].  Workspace: pgica_retrieval_ranks_workspace_bytes() (ceil(rows/256) * ceil(cols/256) + 4 * (rows +
+ * cols) bytes, rounded up). */
+int pgica_retrieval_ranks_workspace_bytes(int64_t rows, int64_t cols, int64_t k, size_t* bytes_host);
+int pgica_retrieval_ranks(const void* a, const void* b, int64_t rows, int64_t cols, int64_t k,
+                          const int32_t* col_owner, int32_t* row_rank, int32_t* col_rank, void* workspace,
+                          size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * K2/K4 core — "softmax-gradient GEMM": the backward of both heads, logits recomputed tile-wise.
  *

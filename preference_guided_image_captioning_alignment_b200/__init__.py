@@ -10,6 +10,7 @@ Drop-in for the loss-head hot path of A-SHOJAEI/preference-guided-image-captioni
     graphs.GraphedCompactDPOStep                            the graphed DPO head on its scored rows only (row buckets)
     distributed.global_ntxent / GlobalContrastiveLoss       NT-Xent with negatives from every rank
     scoring.compute_similarity / paired_scores              retrieval-style scoring on the similarity kernel
+    scoring.retrieval_ranks_both / retrieval_recall         image-text retrieval ranks and recall@k in both directions
     optim.FusedAdamW                                        AdamW with the NaN-safe global-norm clip folded into one update pass
     install()                                               rebinds the reference's names to the above
 
@@ -24,9 +25,11 @@ from .install import fuse_model, install, unfuse_model, uninstall  # noqa: F401
 from .prologue import collapsed_cross_attention_ln, ln_l2norm  # noqa: F401
 from .losses import ContrastiveLoss, DeferredLoss, LazyLogits, PreferenceLoss  # noqa: F401
 from .optim import FusedAdamW  # noqa: F401
-from .scoring import compute_similarity, paired_scores, retrieval_ranks  # noqa: F401
+from .scoring import (compute_similarity, paired_scores, retrieval_ranks, retrieval_ranks_both,  # noqa: F401
+                      retrieval_recall)
 
 __all__ = ["ContrastiveLoss", "PreferenceLoss", "DPOPreferenceLoss", "FusedDPOHead", "TemperatureScaledSimilarity",
            "compute_sequence_logprobs", "lmhead_sequence_logprobs", "LazyLogits", "GraphedDPOStep", "GraphedCompactDPOStep", "GraphedContrastiveStep", "NaNSafeGradientNorm",
            "install", "uninstall", "fuse_model", "unfuse_model", "collapsed_cross_attention_ln", "ln_l2norm", "DeferredLoss", "compute_similarity", "paired_scores", "retrieval_ranks",
+           "retrieval_ranks_both", "retrieval_recall",
            "FusedAdamW"]

@@ -15,6 +15,8 @@
 // round-robin to the persistent pairs, so at any moment the whole grid works on the same four or five B tiles:
 // B (the 103 MB LM-head weight) is then read from HBM once instead of once per row block.  Every tile writes its
 // rows' (max, sum, target) as a partial; lse_merge_kernel folds the column tiles of a row (deterministic, no atomics).
+#include <algorithm>
+
 #include "common.h"
 #include "ptx.cuh"
 
@@ -62,6 +64,40 @@ struct GemmLseParams {
   int cols_pad;
 };
 
+// What the epilogue warps do with a tile.  The two retrieval-rank passes run the same tiles in the same k-order as each
+// other, so a positive's score found in the first pass is bit-identical to the value the second pass compares with.
+enum TileEpilogue : int {
+  kEpiLse = 0,        // online log-sum-exp + target gather (pgica_gemm_lse, pgica_similarity)
+  kEpiLseCols = 1,    // the same plus the column statistics (pgica_gemm_lse_rowcol)
+  kEpiPositives = 2,  // retrieval pass 1: only tiles holding a (owner[j], j) pair; publishes p (rows) and q (columns)
+  kEpiRanks = 3,      // retrieval pass 2: every tile; counts scores above p along rows and above q along columns
+};
+
+// Retrieval ranks (pgica_retrieval_ranks).  Rows are images, columns captions; caption j belongs to row owner(j).
+struct RankParams {
+  const int32_t* col_owner;  // [cols] owner of each column; NULL = column j belongs to row j (j < rows).  Entries outside
+                             // [0, rows) own nothing.
+  uint8_t* tile_mask;        // [num_n_tiles * num_m_pairs], indexed like the tile walk: 1 = the tile holds a positive
+  uint32_t* pos_key;         // [rows] p of the row as an order-preserving key (pos_key_of); 0 = the row owns no column
+  float* pos_col;            // [cols] q of the column; NaN when it has no owner (a NaN threshold counts nothing)
+  int32_t* row_rank;         // [rows] outputs
+  int32_t* col_rank;         // [cols]
+};
+
+// Order-preserving uint32 key of an fp32 score for atomicMax: -inf < ... < -0 < +0 < ... < +inf < NaN, and 0 below all
+// of them, so a row's maximum over several tiles (and pair CTAs) is one integer max that propagates NaN.
+__device__ __forceinline__ uint32_t pos_key_of(float v) {
+  const uint32_t u = __float_as_uint(v);
+  return v != v ? 0xFFFFFFFFu : ((u & 0x80000000u) ? ~u : (u | 0x80000000u));
+}
+__device__ __forceinline__ float pos_value(uint32_t key) {  // key 0 (no positive) decodes to NaN: nothing counts
+  return key == 0xFFFFFFFFu ? NAN : __uint_as_float((key & 0x80000000u) ? (key & 0x7FFFFFFFu) : ~key);
+}
+__device__ __forceinline__ int col_owner_of(const RankParams& r, int rows, int col) {
+  const int o = r.col_owner ? r.col_owner[col] : (col < rows ? col : -1);
+  return (o >= 0 && o < rows) ? o : -1;
+}
+
 __device__ __forceinline__ void tma_load_2d_pair(void* smem_dst, const void* tmap, uint32_t bar_cluster, int c0, int c1) {
   asm volatile(
       "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
@@ -86,11 +122,19 @@ __device__ __forceinline__ void umma2_commit_both(uint64_t* bar) {
 
 constexpr size_t kSmemBytes = 1024 /*align slack*/ + kStages * (kABytes + kBBytes) + 256 /*barriers*/;
 
-template <bool kCols>  // kCols: also publish the column statistics (a separate instantiation: the plain forward keeps its code)
-__global__ void __launch_bounds__(block_threads(kCols), 1)
-gemm_lse_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
-                const GemmLseParams p) {
-  constexpr int kEpiGroups = epi_groups(kCols);
+template <bool kPositives>
+__device__ __forceinline__ void rank_epilogue(const GemmLseParams& p, const RankParams& r, int warp, int lane, uint32_t rho,
+                                              uint32_t tmem_base, uint64_t* tfull_bar, uint64_t* tempty_bar, int t_begin,
+                                              int t_step, int t_end);
+
+// The tile pipeline of every kernel in this file: barrier and TMEM set-up, the TMA producers, the MMA issuer, the
+// epilogue selected by kMode, teardown.  In kEpiPositives every role skips the tiles tile_mask leaves out before any TMA
+// or MMA, so their ring and accumulator phases stay in step.
+template <int kMode>
+__device__ __forceinline__ void gemm_tiles(const CUtensorMap& tm_a, const CUtensorMap& tm_b, const GemmLseParams p,
+                                           const RankParams r) {
+  constexpr bool kCols = kMode == kEpiLseCols;
+  constexpr int kEpiGroups = epi_groups(kMode != kEpiLse);
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = align_smem_1024(smem_raw);
   uint8_t* smem_a = smem;
@@ -144,6 +188,9 @@ gemm_lse_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
     uint32_t phase = 0, stage_no = 0;
     const uint32_t lbar0 = mapa_u32(smem_u32(&full_bar[0]), 0);  // the leader's full barriers (shared::cluster)
     for (int t = t_begin; t < t_end; t += t_step) {
+      if constexpr (kMode == kEpiPositives) {
+        if (!r.tile_mask[t]) continue;
+      }
       const int n_tile = t / p.num_m_pairs;
       const int m_blk = 2 * (t - n_tile * p.num_m_pairs) + (int)rho;
       for (int kb = 0; kb < num_kb; ++kb, ++stage_no) {
@@ -171,6 +218,9 @@ gemm_lse_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
     int stage = 0, acc = 0;
     uint32_t phase = 0, acc_phase = 0;
     for (int t = t_begin; t < t_end; t += t_step) {
+      if constexpr (kMode == kEpiPositives) {
+        if (!r.tile_mask[t]) continue;
+      }
       mbar_wait_cluster(&tempty_bar[acc], acc_phase ^ 1);
       tc_fence_after_sync();
       const uint32_t d_tmem = tmem_base + acc * kBlockN;
@@ -197,7 +247,11 @@ gemm_lse_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
         acc_phase ^= 1;
       }
     }
-  } else if (warp >= kEpilogueWarp0) {
+  } else if (warp < kEpilogueWarp0) {
+    // warp 1 of the second CTA, warp 3: idle
+  } else if constexpr (kMode >= kEpiPositives) {
+    rank_epilogue<kMode == kEpiPositives>(p, r, warp, lane, rho, tmem_base, tfull_bar, tempty_bar, t_begin, t_step, t_end);
+  } else {
     const int quarter = warp & 3;  // TMEM lane quarter this warp may read
     const int wg = (warp - kEpilogueWarp0) >> 2;  // column group of the tile
     constexpr int kChunks = kBlockN / 32 / kEpiGroups;
@@ -323,6 +377,137 @@ gemm_lse_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
                  : "memory");
 }
 
+template <bool kCols>  // kCols: also publish the column statistics (a separate instantiation: the plain forward keeps its code)
+__global__ void __launch_bounds__(block_threads(kCols), 1)
+gemm_lse_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
+                const GemmLseParams p) {
+  gemm_tiles<kCols ? kEpiLseCols : kEpiLse>(tm_a, tm_b, p, RankParams{});
+}
+
+// Retrieval ranks, pass 1 (kPositives) and pass 2: the same tile pipeline with the rank-counting epilogue.
+template <bool kPositives>
+__global__ void __launch_bounds__(block_threads(true), 1)
+gemm_rank_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
+                 const GemmLseParams p, const RankParams r) {
+  gemm_tiles<kPositives ? kEpiPositives : kEpiRanks>(tm_a, tm_b, p, r);
+}
+
+// Epilogue of the rank passes: 8 warps, warp w reads TMEM lane quarter w & 3 (32 rows) and column half (w - 4) >> 2.
+//   pass 1: per 32-column chunk every lane holds the owner of its column; the row that owns column j keeps the running
+//           max of its positives (one atomicMax of the key per tile) and stores q[j] (exactly one writer per column).
+//   pass 2: rows count their scores above p in a per-thread counter over the tile's chunks; columns are counted per
+//           chunk with one ballot per column (the warp's 32 rows against lane j's q) and one popc.  Both are added to the
+//           int32 outputs with red.global.add: exact and order-independent.
+template <bool kPositives>
+__device__ __forceinline__ void rank_epilogue(const GemmLseParams& p, const RankParams& r, int warp, int lane, uint32_t rho,
+                                              uint32_t tmem_base, uint64_t* tfull_bar, uint64_t* tempty_bar, int t_begin,
+                                              int t_step, int t_end) {
+  constexpr int kChunks = kBlockN / 32 / 2;
+  const int quarter = warp & 3;
+  const int wg = (warp - kEpilogueWarp0) >> 2;
+  const int row_in_blk = quarter * 32 + lane;
+  int acc = 0;
+  uint32_t acc_phase = 0;
+  for (int t = t_begin; t < t_end; t += t_step) {
+    if (kPositives && !r.tile_mask[t]) continue;
+    const int n_tile = t / p.num_m_pairs;
+    const int m_blk = 2 * (t - n_tile * p.num_m_pairs) + (int)rho;  // may be one past the end (odd block count)
+    const int row = m_blk * kBlockM + row_in_blk;
+    const bool rvalid = row < p.rows;
+    const int n0 = n_tile * kBlockN;
+    uint32_t key = 0;
+    if (!kPositives && rvalid) key = r.pos_key[row];
+    const float thr = pos_value(key);
+    int row_count = 0;
+    mbar_wait(&tfull_bar[acc], acc_phase);
+    tc_fence_after_sync();
+    const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + acc * kBlockN;
+#pragma unroll 1
+    for (int cl = 0; cl < kChunks; ++cl) {
+      const int c0 = n0 + (wg * kChunks + cl) * 32;
+      if (c0 >= p.cols) break;  // warp-uniform: nothing valid from here on
+      const int col = c0 + lane;
+      int own = -1;
+      float q = NAN;
+      if (col < p.cols) {
+        if (kPositives)
+          own = col_owner_of(r, p.rows, col);
+        else
+          q = r.pos_col[col];
+      }
+      uint32_t u[32];
+      tmem_ld_32x32(taddr + (c0 - n0), u);
+      tmem_ld_wait();
+      float v[32];
+#pragma unroll
+      for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(u[j]);
+      if (c0 + 32 > p.cols) {
+#pragma unroll
+        for (int j = 0; j < 32; ++j)
+          if (c0 + j >= p.cols) v[j] = -INFINITY;  // above no threshold
+      }
+      if (kPositives) {
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+          if (__shfl_sync(0xffffffffu, own, j) == row) {  // own is -1 or < rows: rows past the end never match
+            key = max(key, pos_key_of(v[j]));
+            r.pos_col[c0 + j] = v[j];
+          }
+        }
+      } else {
+        uint32_t mine = 0;  // ballot over the warp's rows for this lane's column
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+          row_count += v[j] > thr ? 1 : 0;
+          const float qj = __shfl_sync(0xffffffffu, q, j);  // every lane, rows past the end included
+          const uint32_t b = __ballot_sync(0xffffffffu, rvalid && v[j] > qj);
+          if (lane == j) mine = b;
+        }
+        const int cc = __popc(mine);
+        if (cc != 0) atomicAdd(&r.col_rank[col], cc);  // q is NaN past the last column: cc == 0 there
+      }
+    }
+    tc_fence_before_sync();
+    mbar_arrive_cluster(&tempty_bar[acc], 0);  // tell the leader: this CTA has read the accumulator
+    if (++acc == kAccStages) {
+      acc = 0;
+      acc_phase ^= 1;
+    }
+    if (kPositives) {
+      if (key != 0) atomicMax(&r.pos_key[row], key);
+    } else if (rvalid) {
+      if (key == 0) {
+        if (n_tile == 0 && wg == 0) r.row_rank[row] = -1;  // owns no column: no tile adds to it
+      } else if (row_count != 0) {
+        atomicAdd(&r.row_rank[row], row_count);
+      }
+    }
+  }
+}
+
+// Retrieval set-up, launch 1 of 2: clear the tile mask, the row keys and the row counts.
+__global__ void rank_init_kernel(const GemmLseParams p, const RankParams r, int mask_bytes) {
+  const int n = mask_bytes > p.rows ? mask_bytes : p.rows;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    if (i < mask_bytes) r.tile_mask[i] = 0;
+    if (i < p.rows) {
+      r.pos_key[i] = 0;
+      r.row_rank[i] = 0;
+    }
+  }
+}
+
+// Launch 2 of 2, one thread per column: range-check the owner, mark the tile that holds (owner[j], j), clear q[j] and the
+// column count (-1 for a column without an owner, which no pass touches again).
+__global__ void rank_mark_kernel(const GemmLseParams p, const RankParams r) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= p.cols) return;
+  const int o = col_owner_of(r, p.rows, j);
+  r.pos_col[j] = NAN;
+  r.col_rank[j] = o >= 0 ? 0 : -1;
+  if (o >= 0) r.tile_mask[(j / kBlockN) * p.num_m_pairs + o / (2 * kBlockM)] = 1;
+}
+
 // Fold the column-tile partials of every row into lse (natural log) and the target logit.  A block handles 32 rows
 // with 8 threads per row: thread (r, g) walks tiles g, g+8, ... (loads coalesced across r), then the 8 running
 // (max, sum, target) triples of a row are combined in a fixed order through shared memory.
@@ -436,6 +621,34 @@ size_t col_stats_bytes(const GemmLseParams& p, size_t* sum_bytes) {
   return *sum_bytes + align_up(groups * (size_t)p.num_n_tiles * 8 * sizeof(float), 256);
 }
 
+// Launch one of the tile kernels on CTA pairs (2-CTA clusters) with the full shared-memory ring.
+template <class Kernel, class... Args>
+int launch_pairs(Kernel kern, int grid, int threads, cudaStream_t st, const Args&... args) {
+  PGICA_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3((unsigned)grid);
+  cfg.blockDim = dim3((unsigned)threads);
+  cfg.dynamicSmemBytes = kSmemBytes;
+  cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 2;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  PGICA_CUDA_OK(cudaLaunchKernelEx(&cfg, kern, args...));
+  count_launches(1);
+  return PGICA_OK;
+}
+
+// Workspace of the retrieval ranks: tile mask, row keys, column positives.  Nothing grows with rows * cols but the mask.
+size_t rank_ws_bytes(const GemmLseParams& p, size_t* mask_bytes, size_t* key_bytes) {
+  *mask_bytes = align_up((size_t)p.num_m_pairs * p.num_n_tiles, 256);
+  *key_bytes = align_up((size_t)p.rows * sizeof(uint32_t), 256);
+  return *mask_bytes + *key_bytes + align_up((size_t)p.cols * sizeof(float), 256);
+}
+
 }  // namespace
 }  // namespace pgica
 
@@ -488,22 +701,9 @@ static int gemm_lse_impl(const void* a, const void* b, int64_t rows, int64_t col
   if (rc != PGICA_OK) return rc;
 
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  auto kern = lse_col ? gemm_lse_kernel<true> : gemm_lse_kernel<false>;
-  PGICA_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(lse_col ? block_threads(true) : block_threads(false));
-  cfg.dynamicSmemBytes = kSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  PGICA_CUDA_OK(cudaLaunchKernelEx(&cfg, kern, tm_a, tm_b, p));
-  count_launches(1);
+  rc = launch_pairs(lse_col ? gemm_lse_kernel<true> : gemm_lse_kernel<false>, grid, block_threads(lse_col != nullptr), st,
+                    tm_a, tm_b, p);
+  if (rc != PGICA_OK) return rc;
   lse_merge_kernel<<<(unsigned)ceil_div(rows, kMergeRows), kMergeRows * kMergeGroups, 0, st>>>(p, lse, tgt);
   PGICA_CUDA_OK(cudaGetLastError());
   count_launches(1);
@@ -540,6 +740,61 @@ int pgica_gemm_lse(const void* a, const void* b, int64_t rows, int64_t cols, int
                    size_t workspace_bytes, void* stream) {
   return gemm_lse_impl(a, b, rows, cols, k, scale, labels, diag_offset, lse, tgt, nullptr, workspace,
                        workspace_bytes, stream);
+}
+
+int pgica_retrieval_ranks_workspace_bytes(int64_t rows, int64_t cols, int64_t k, size_t* bytes_host) {
+  pgica::GemmLseParams p{};
+  int grid = 0;
+  size_t lse_bytes = 0, mask_bytes = 0, key_bytes = 0;
+  int rc = pgica::plan(rows, cols, k, &p, &grid, &lse_bytes);
+  if (rc != PGICA_OK) return rc;
+  PGICA_REQUIRE(bytes_host, "workspace query: null result pointer");
+  *bytes_host = pgica::rank_ws_bytes(p, &mask_bytes, &key_bytes);
+  return PGICA_OK;
+}
+
+int pgica_retrieval_ranks(const void* a, const void* b, int64_t rows, int64_t cols, int64_t k, const int32_t* col_owner,
+                          int32_t* row_rank, int32_t* col_rank, void* workspace, size_t workspace_bytes, void* stream) {
+  using namespace pgica;
+  int rc = pgica_device_check();
+  if (rc != PGICA_OK) return rc;
+  GemmLseParams p{};
+  int grid = 0;
+  size_t lse_bytes = 0, mask_bytes = 0, key_bytes = 0;
+  rc = plan(rows, cols, k, &p, &grid, &lse_bytes);
+  if (rc != PGICA_OK) return rc;
+  PGICA_REQUIRE(a && b && row_rank && col_rank, "retrieval_ranks: null operand");
+  const size_t need = rank_ws_bytes(p, &mask_bytes, &key_bytes);
+  if (workspace_bytes < need || !workspace) {
+    set_error("retrieval_ranks: workspace too small (%zu < %zu)", workspace_bytes, need);
+    return PGICA_ERR_WORKSPACE_TOO_SMALL;
+  }
+  RankParams r{};
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  r.col_owner = col_owner;
+  r.tile_mask = ws;
+  r.pos_key = reinterpret_cast<uint32_t*>(ws + mask_bytes);
+  r.pos_col = reinterpret_cast<float*>(ws + mask_bytes + key_bytes);
+  r.row_rank = row_rank;
+  r.col_rank = col_rank;
+
+  CUtensorMap tm_a, tm_b;
+  rc = make_tmap_bf16(&tm_a, a, rows, k, k, kBlockM);
+  if (rc != PGICA_OK) return rc;
+  rc = make_tmap_bf16(&tm_b, b, cols, k, k, kBlockN / 2);
+  if (rc != PGICA_OK) return rc;
+
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int64_t init_n = std::max<int64_t>((int64_t)(p.num_m_pairs * p.num_n_tiles), rows);
+  rank_init_kernel<<<(unsigned)std::min<int64_t>(ceil_div(init_n, 256), 4096), 256, 0, st>>>(p, r, p.num_m_pairs * p.num_n_tiles);
+  PGICA_CUDA_OK(cudaGetLastError());
+  count_launches(1);
+  rank_mark_kernel<<<(unsigned)ceil_div(cols, 256), 256, 0, st>>>(p, r);
+  PGICA_CUDA_OK(cudaGetLastError());
+  count_launches(1);
+  rc = launch_pairs(gemm_rank_kernel<true>, grid, block_threads(true), st, tm_a, tm_b, p, r);
+  if (rc != PGICA_OK) return rc;
+  return launch_pairs(gemm_rank_kernel<false>, grid, block_threads(true), st, tm_a, tm_b, p, r);
 }
 
 int pgica_similarity(const void* a, const void* b, int64_t rows, int64_t cols, int64_t k, float scale, float* sim,

@@ -90,6 +90,23 @@ def similarity(a, b, scale=1.0):
     return sim
 
 
+def retrieval_ranks(a, b, col_owner=None):
+    """(row_rank int32 (rows,), col_rank int32 (cols,)) of pgica_retrieval_ranks; a, b bf16 [*, k], col_owner int32
+    (cols,) or None (caption j belongs to image j)."""
+    _need_cuda(a, b, col_owner)
+    lib = _lib.load()
+    rows, k = a.shape
+    cols = b.shape[0]
+    need = ctypes.c_size_t(0)
+    _lib.check(lib.pgica_retrieval_ranks_workspace_bytes(rows, cols, k, ctypes.byref(need)))
+    ws = _ws(need.value, a.device)
+    row_rank = torch.empty(rows, dtype=torch.int32, device=a.device)
+    col_rank = torch.empty(cols, dtype=torch.int32, device=a.device)
+    _lib.check(lib.pgica_retrieval_ranks(_p(a), _p(b), rows, cols, k, _p(col_owner), _p(row_rank), _p(col_rank), _p(ws),
+                                         need.value, _stream()))
+    return row_rank, col_rank
+
+
 # ----------------------------------------------------------------------------------------- K2/K4 core
 def softmax_grad_gemm(x, y, scale=1.0, row=None, col=None, out_dtype=torch.float32):
     """out = G(x y^T) y with G built from row stats (lse, coef, tgt) and/or column stats (see pgica.h)."""
